@@ -2,6 +2,7 @@
 """bench.py -- denoise-steps/s of the SDXL + IMAGHarmony hot path (BASELINE.json metric) on N GPUs of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--images n] [--res 1024]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: UNet forward on the CFG pair(s) + CFG combine + Euler update
 (custom_pipelines.py:325-363) at 1024x1024 (latent 128x128), random-init SDXL-base weights, synthetic embeddings.
@@ -20,6 +21,9 @@ A "step" is one pass of the hot path over one batch: UNet forward on the CFG pai
   cpu_baseline : the CPU oracle (a port of the reference's PyTorch path) on the host cores, bounded sample
   pns (N > 1) : BASELINE config 4 shape -- 4 candidates per GPU, K steps each, H2D + denoise + score + all_gather +
           winner broadcast, wall clock max over ranks, against the bar 1.1 x 4 x (single-candidate time)
+`--dump-outputs DIR` writes the final latents of the timed steps (what `DenoiseEngine.run` returns) to DIR/latents.npy
+(DIR/latents_rank<r>.npy with N > 1 ranks) in float32: weights and inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 `--impl reference` times the CPU path alone (rank 0 only): every step is one REAL denoise step (UNet on the CFG pair +
 CFG + Euler) of the oracle at the largest of 512^2 / 384^2 / 256^2 that keeps the K + W steps within the time budget.
 """
@@ -119,6 +123,23 @@ def synth_inputs(cfg, n: int, lat: int, T: int, rank: int):
     res = lat * 8.0
     tid = torch.tensor([[res, res, 0.0, 0.0, res, res]] * n)
     return latents, pos, neg, pooled, npooled, tid
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, arrays: dict) -> None:
+    """DIR/<name>.npy in float32.  An array larger than the 64 MB budget is written as a fixed, seeded sample of its
+    flattened elements (the same positions on every run), so the dump stays comparable at any batch or resolution."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    keep = DUMP_LIMIT_BYTES // 4 // max(len(arrays), 1)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if a.numel() > keep:
+            idx = torch.randperm(a.numel(), generator=torch.Generator("cpu").manual_seed(0))[:keep].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(directory, f"{name}.npy"), a.numpy())
 
 
 def workload_string(res: int, steps: int, images: int) -> str:
@@ -625,7 +646,13 @@ def main():
                          "bigG towers + SDXL VAE) or the synthetic linear probe of the latent")
     ap.add_argument("--pns-preview", type=int, default=0,
                     help="two-phase PNS: preview steps per candidate before the judge; the winner alone runs the rest")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the final latents of the timed steps to DIR/latents.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or args.pns > 0):
+        ap.error("--dump-outputs records the timed denoise steps of the native path; not with --impl reference or --pns")
 
     if args.impl == "reference":
         run_reference_arm(args)
@@ -695,6 +722,8 @@ def main():
         barrier()
     dev_s = ev0.elapsed_time(ev2) * 1e-3
     tail_ms = ev1.elapsed_time(ev2)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"latents" if world == 1 else f"latents_rank{rank}": st["latents"]})
 
     # ---- end to end through the public API: pinned host inputs -> H2D -> K steps -> D2H of the result -------------
     barrier()

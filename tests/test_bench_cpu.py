@@ -92,6 +92,22 @@ def test_peaks_come_from_the_driver_file_when_present():
         assert pk["source"].startswith("measured")
 
 
+def test_dump_outputs_writes_float32_and_samples_past_the_budget(tmp_path, monkeypatch):
+    """`--dump-outputs`: DIR/<name>.npy in float32, whole when it fits; past the budget a seeded sample that is the same
+    on every call."""
+    import numpy as np
+    x = torch.randn(2, 4, 8, 8, generator=torch.Generator("cpu").manual_seed(5)).half()
+    bench.dump_outputs(str(tmp_path / "d"), {"latents": x})
+    a = np.load(tmp_path / "d" / "latents.npy")
+    assert a.dtype == np.float32 and a.shape == (2, 4, 8, 8) and np.array_equal(a, x.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 100 * 4)
+    bench.dump_outputs(str(tmp_path / "s1"), {"latents": x})
+    bench.dump_outputs(str(tmp_path / "s2"), {"latents": x})
+    s1, s2 = np.load(tmp_path / "s1" / "latents.npy"), np.load(tmp_path / "s2" / "latents.npy")
+    assert s1.dtype == np.float32 and s1.shape == (100,) and np.array_equal(s1, s2)
+    assert np.isin(s1, x.float().numpy().reshape(-1)).all()
+
+
 def test_reference_arm_line_schema(monkeypatch, capsys):
     """`bench.py --impl reference`: one JSON line with the contract's keys; rank != 0 prints nothing."""
     monkeypatch.setattr(bench, "CpuOracle", lambda: _FakeOracle(0.5))

@@ -60,22 +60,14 @@ def test_convert_bin_tool(tmp_path, capsys):
 
 
 def test_convert_bin_tool_agrees_with_the_reference_tool(tmp_path, capsys):
-    """Where the reference tree is on disk (this container, not the GPU box): the reference's own converter and ours
-    write the same file for the same training checkpoint."""
-    import importlib.util
-    import pytest
-    ref_path = "/root/reference/convert_bin.py"
-    if not os.path.exists(ref_path):
-        pytest.skip("reference tree not present")
+    """The reference's own converter and ours write the same file for the same training checkpoint (the reference's
+    output is tests/golden/reference_helpers.pt, written by oracle/make_helper_goldens.py)."""
     import convert_bin
-    spec = importlib.util.spec_from_file_location("reference_convert_bin", ref_path)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    gold = torch.load(os.path.join(os.path.dirname(__file__), "golden", "reference_helpers.pt"), map_location="cpu")
     src = tmp_path / "pytorch_model.bin"
-    torch.save(_flat_training_checkpoint(), src)
-    assert ref.convert_checkpoint_to_ip_adapter(str(src), str(tmp_path / "ref.bin")) is True
+    torch.save(gold["convert_bin"]["checkpoint"], src)
     assert convert_bin.convert_checkpoint_to_ip_adapter(str(src), str(tmp_path / "own.bin")) is True
-    a, b = torch.load(tmp_path / "ref.bin", map_location="cpu"), torch.load(tmp_path / "own.bin", map_location="cpu")
+    a, b = gold["convert_bin"]["converted"], torch.load(tmp_path / "own.bin", map_location="cpu")
     assert list(a) == list(b)
     for part in a:
         assert list(a[part]) == list(b[part])

@@ -16,7 +16,8 @@ GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "reference_vectors.pt
 
 @pytest.fixture(scope="module")
 def gold():
-    return torch.load(GOLDEN, map_location="cpu")
+    from oracle.check_against_reference import load_golden
+    return load_golden(GOLDEN)
 
 
 def test_ip_attn_processor_matches_reference(gold):

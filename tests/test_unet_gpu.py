@@ -66,7 +66,8 @@ def test_native_processors_match_reference_goldens():
     """IPAttnProcessor2_0 / AttnProcessor2_0 on the kernels vs outputs of the reference's own classes."""
     from imagharmony_b200.unet import Attention
     from ip_adapter.attention_processor import AttnProcessor2_0, IPAttnProcessor2_0
-    gold = torch.load(GOLDEN, map_location="cpu")
+    from oracle.check_against_reference import load_golden
+    gold = load_golden(GOLDEN)
     for skip in (0, 1):
         g = gold[f"ipattn_skip{skip}"]
         C, D = g["hidden"].shape[-1], g["ehs"].shape[-1]
@@ -190,7 +191,8 @@ def test_adapter_modules_match_reference_goldens_on_gpu():
     (train.py:188-266, ip_adapter.py:28-48, resampler.py:81-147), parameters and inputs rounded to fp16."""
     from imagharmony_b200 import adapter as N
     from oracle import adapter_ref as A
-    gold = torch.load(GOLDEN, map_location="cpu")
+    from oracle.check_against_reference import load_golden
+    gold = load_golden(GOLDEN)
 
     def h(sd):
         return {k: v.half() for k, v in sd.items()}
