@@ -72,6 +72,8 @@ SIGNATURES = {
                                      c_int, c_float, c_void_p]),
     "ih_conv2d_shortcut_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_void_p, c_int, c_void_p, c_int,
                                        c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "ih_conv2d_s2_padbr_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
+                                       c_void_p]),
     "ih_gemm_set_trace": (None, [c_void_p]),
     "ih_gemm_prefetch_next": (None, [c_void_p, c_longlong]),
     "ih_conv2d_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_void_p, c_void_p, c_int, c_int,
@@ -105,6 +107,9 @@ SIGNATURES = {
     "ih_conv_in_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "ih_conv_out_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "ih_im2col3x3_nchw_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "ih_image_im2col3x3_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
+    "ih_vae_sample_add_noise_f16": (c_int, [c_void_p, c_longlong, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int,
+                                            c_int, c_int, c_int, c_float, c_float, c_void_p]),
     "ih_nhwc_to_nchw_f16": (c_int, [c_void_p, c_longlong, c_void_p, c_int, c_longlong, c_int, c_void_p]),
     "ih_euler_cfg_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_longlong, c_int,
                                   c_void_p]),

@@ -70,7 +70,7 @@ HARMONY_TINY = HarmonyConfig(image_hidden_size=64, text_context_dim=128, inter_d
 
 @dataclass(frozen=True)
 class VAEConfig:
-    """[3P] diffusers AutoencoderKL of SDXL (decoder half): vae/config.json of stabilityai/stable-diffusion-xl-base-1.0."""
+    """[3P] diffusers AutoencoderKL of SDXL (decoder and encoder): vae/config.json of stabilityai/stable-diffusion-xl-base-1.0."""
     latent_channels: int = 4
     out_channels: int = 3
     block_out_channels: Tuple[int, ...] = (128, 256, 512, 512)
@@ -80,6 +80,7 @@ class VAEConfig:
     sample_size: int = 1024               # tiling: tiles of sample_size pixels (= sample_size / 8 latents), 25 % overlap
     tile_overlap_factor: float = 0.25
     force_upcast: bool = True             # vae/config.json of SDXL-base: the reference upcasts the VAE to fp32 (custom_pipelines.py:366-371)
+    in_channels: int = 3                  # image channels the encoder reads (img2img)
 
     @property
     def tile_latent_min_size(self) -> int:

@@ -937,7 +937,7 @@ static int gemm_impl(const void* a, long long lda, const void* w, const void* bi
 static int conv_impl(const void* x, const void* w, const void* bias, const void* rowbias, long long ld_rowbias,
                      const void* residual, void* out, int B, int Hin, int Win, int Cin, int Cout, int ksize, int stride,
                      int tile_n, float alpha, void* stream, const void* sc0 = nullptr, int Csc0 = 0,
-                     const void* sc1 = nullptr, int Csc1 = 0);
+                     const void* sc1 = nullptr, int Csc1 = 0, bool pad_br = false);
 
 extern "C" int ih_conv2d_f16(const void* x, const void* w, const void* bias, const void* rowbias,
                              long long ld_rowbias, const void* residual, void* out, int B, int Hin, int Win, int Cin,
@@ -951,6 +951,12 @@ extern "C" int ih_conv2d_scaled_f16(const void* x, const void* w, const void* bi
   return conv_impl(x, w, bias, nullptr, 0, residual, out, B, Hin, Win, Cin, Cout, 3, stride, 0, alpha, stream);
 }
 
+extern "C" int ih_conv2d_s2_padbr_f16(const void* x, const void* w, const void* bias, void* out, int B, int Hin, int Win,
+                                      int Cin, int Cout, void* stream) {
+  return conv_impl(x, w, bias, nullptr, 0, nullptr, out, B, Hin, Win, Cin, Cout, 3, 2, 0, 1.f, stream, nullptr, 0, nullptr,
+                   0, true);
+}
+
 extern "C" int ih_conv2d_shortcut_f16(const void* x, const void* w, const void* bias, const void* rowbias,
                                       long long ld_rowbias, const void* sc0, int Csc0, const void* sc1, int Csc1, void* out,
                                       int B, int H, int W, int Cin, int Cout, void* stream) {
@@ -962,7 +968,8 @@ extern "C" int ih_conv2d_shortcut_f16(const void* x, const void* w, const void* 
 
 static int conv_impl(const void* x, const void* w, const void* bias, const void* rowbias, long long ld_rowbias,
                      const void* residual, void* out, int B, int Hin, int Win, int Cin, int Cout, int ksize, int stride,
-                     int tile_n, float alpha, void* stream, const void* sc0, int Csc0, const void* sc1, int Csc1) {
+                     int tile_n, float alpha, void* stream, const void* sc0, int Csc0, const void* sc1, int Csc1,
+                     bool pad_br) {
   const PrefetchHint hint = take_prefetch_hint();
   IH_CHECK(x && w && out, IH_ERR_ARG, "ih_conv2d_f16: null pointer");
   IH_CHECK(ksize == 3, IH_ERR_ARG, "ih_conv2d_f16: ksize must be 3 (1x1 convs are ih_gemm_f16)");
@@ -1044,7 +1051,9 @@ static int conv_impl(const void* x, const void* w, const void* bias, const void*
     }
   } else {
     IH_CHECK(!sc0, IH_ERR_ARG, "ih_conv2d: a fused shortcut needs stride 1");
-    // input row 2*oy + dy - 1: dy=0 -> odd rows at oy-1, dy=1 -> even rows at oy, dy=2 -> odd rows at oy
+    // padding 1: input row 2*oy + dy - 1: dy=0 -> odd rows at oy-1, dy=1 -> even rows at oy, dy=2 -> odd rows at oy.
+    // pad_br (bottom / right padding only): input row 2*oy + dy: dy=0 -> even rows at oy, dy=1 -> odd rows at oy,
+    // dy=2 -> even rows at oy+1, which is out of bounds on the last output row and column: TMA fills it with zeros.
     for (int py = 0; py < 2; ++py)
       for (int px = 0; px < 2; ++px) {
         const __half* base = (const __half*)x + ((long long)py * Win + px) * Cin;
@@ -1053,8 +1062,8 @@ static int conv_impl(const void* x, const void* w, const void* bias, const void*
         int rc = get_tmap_f16(&amaps.m[py * 2 + px], base, 4, adims, astr, abox);
         if (rc) return rc;
       }
-    const int par[3] = {1, 0, 1};
-    const int off[3] = {-1, 0, 0};
+    const int par[3] = {pad_br ? 0 : 1, pad_br ? 1 : 0, pad_br ? 0 : 1};
+    const int off[3] = {pad_br ? 0 : -1, 0, pad_br ? 1 : 0};
     for (int t = 0; t < 9; ++t) {
       const int dy = t / 3, dx = t % 3;
       p.tap_map[t] = (signed char)(par[dy] * 2 + par[dx]);

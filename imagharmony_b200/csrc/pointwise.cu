@@ -711,6 +711,74 @@ __global__ void nhwc_to_nchw_kernel(const __half* __restrict__ x, long long ldc,
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// The two ends of the VAE encoder (img2img):
+//   image front end: uint8 RGB NHWC (the PIL pixels) -> im2col rows [B*H*W, Kpad] of the normalised image for the
+//                    encoder's conv_in GEMM.  Value = fp16(2 * (v / 255) - 1) with diffusers' fp32 rounding points
+//                    (numpy `/ 255.0` in fp32, then `2 * x - 1` in fp32), zero padding 1, zero K padding.
+//   sample + noise : z = fp16(sf * fp16(mean + exp(0.5 clamp(logvar, -30, 20)) * eps))  (DiagonalGaussianDistribution
+//                    .sample in fp32, the cast to fp16, `scaling_factor * latents` in fp16), then
+//                    fp16(z + fp16(noise * fp16(sigma)))  (EulerDiscreteScheduler.add_noise on fp16 tensors).
+// ---------------------------------------------------------------------------------------------------------------
+__global__ void image_im2col3x3_u8_kernel(const unsigned char* __restrict__ x, __half* __restrict__ out, int B, int H,
+                                          int W, int Kpad) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const long long npix = (long long)B * H * W;
+  const int kv = Kpad >> 3;
+  const long long total = npix * kv;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int v = (int)(i % kv);
+    const long long pix = i / kv;
+    const int xw = (int)(pix % W);
+    const int yh = (int)((pix / W) % H);
+    const int b = (int)(pix / ((long long)W * H));
+    __align__(16) __half vals[8];
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+      const int k = v * 8 + e;
+      __half hv = __float2half_rn(0.f);
+      if (k < 27) {
+        const int ci = k / 9, t = k - ci * 9;
+        const int yy = yh + t / 3 - 1, xx = xw + t % 3 - 1;
+        if (yy >= 0 && yy < H && xx >= 0 && xx < W) {
+          const float u = (float)x[(((long long)b * H + yy) * W + xx) * 3 + ci];
+          hv = __float2half_rn(__fsub_rn(__fmul_rn(2.f, __fdiv_rn(u, 255.f)), 1.f));
+        }
+      }
+      vals[e] = hv;
+    }
+    *reinterpret_cast<uint4*>(out + pix * Kpad + v * 8) = *reinterpret_cast<const uint4*>(vals);
+  }
+}
+
+__global__ void vae_sample_add_noise_kernel(const __half* __restrict__ moments, long long ldm, int Bm,
+                                            const float* __restrict__ eps, int Be, const __half* __restrict__ noise,
+                                            __half* __restrict__ out, int B, int C, long long HW, float sf, float sigma) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const float sig16 = __half2float(__float2half_rn(sigma));
+  const long long total = (long long)B * C * HW;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const long long p = i % HW;
+    const int c = (int)((i / HW) % C);
+    const int b = (int)(i / (HW * C));
+    const __half* m = moments + ((long long)(b % Bm) * HW + p) * ldm;
+    float z;
+    if (eps) {
+      const float lv = fminf(fmaxf(__half2float(m[C + c]), -30.f), 20.f);
+      const float sd = expf(0.5f * lv);
+      const float e = eps[((long long)(b % Be) * C + c) * HW + p];
+      const float smp = __fadd_rn(__half2float(m[c]), __fmul_rn(sd, e));
+      z = __half2float(__float2half_rn(__fmul_rn(__half2float(__float2half_rn(smp)), sf)));
+    } else {
+      z = __half2float(m[c]);                        // latents given as they are (4-channel image input)
+    }
+    const float ns = __half2float(__float2half_rn(__fmul_rn(__half2float(noise[i]), sig16)));
+    out[i] = __float2half_rn(__fadd_rn(z, ns));
+  }
+}
+
 static int grid_for(long long total, int threads) {
   long long b = (total + threads - 1) / threads;
   const long long cap = (long long)num_sms() * 16;
@@ -942,5 +1010,29 @@ extern "C" int ih_nhwc_to_nchw_f16(const void* x, long long ldc, void* out, int 
   const long long total = (long long)B * C * HW;
   IH_CUDA(launch_kernel(nhwc_to_nchw_kernel, dim3(grid_for(total, 256)), dim3(256), (size_t)0, (cudaStream_t)stream,
                         (const __half*)x, ldc, (__half*)out, B, HW, C));
+  return 0;
+}
+
+extern "C" int ih_image_im2col3x3_u8(const void* rgb_u8, void* out, int B, int H, int W, int Kpad, void* stream) {
+  IH_CHECK(rgb_u8 && out, IH_ERR_ARG, "ih_image_im2col3x3_u8: null pointer");
+  IH_CHECK(B > 0 && H > 0 && W > 0 && Kpad % 8 == 0 && Kpad >= 27, IH_ERR_SHAPE, "ih_image_im2col3x3_u8: bad shape");
+  const long long total = (long long)B * H * W * (Kpad / 8);
+  IH_CUDA(launch_kernel(image_im2col3x3_u8_kernel, dim3(grid_for(total, 256)), dim3(256), (size_t)0, (cudaStream_t)stream,
+                        (const unsigned char*)rgb_u8, (__half*)out, B, H, W, Kpad));
+  return 0;
+}
+
+extern "C" int ih_vae_sample_add_noise_f16(const void* moments, long long ldm, int Bm, const void* eps_f32, int Be,
+                                           const void* noise, void* out_nchw, int B, int C, int h, int w,
+                                           float scaling_factor, float sigma, void* stream) {
+  IH_CHECK(moments && noise && out_nchw, IH_ERR_ARG, "ih_vae_sample_add_noise_f16: null pointer");
+  IH_CHECK(B > 0 && C > 0 && h > 0 && w > 0 && Bm > 0 && B % Bm == 0 && ldm >= (eps_f32 ? 2 * C : C), IH_ERR_SHAPE,
+           "ih_vae_sample_add_noise_f16: bad shape (B %% Bm == 0 and ldm >= 2C with eps, >= C without are required)");
+  IH_CHECK(!eps_f32 || (Be > 0 && B % Be == 0), IH_ERR_SHAPE, "ih_vae_sample_add_noise_f16: B %% Be != 0");
+  const long long HW = (long long)h * w;
+  const long long total = (long long)B * C * HW;
+  IH_CUDA(launch_kernel(vae_sample_add_noise_kernel, dim3(grid_for(total, 256)), dim3(256), (size_t)0, (cudaStream_t)stream,
+                        (const __half*)moments, ldm, Bm, (const float*)eps_f32, Be, (const __half*)noise,
+                        (__half*)out_nchw, B, C, HW, scaling_factor, sigma));
   return 0;
 }

@@ -92,7 +92,7 @@ class DenoiseEngine:
             control_guidance_start: float = 0.0, control_guidance_end: float = 1.0, stop_after: Optional[int] = None,
             start_step: int = 0, guidance_rescale: float = 0.0, num_loop_steps: Optional[int] = None,
             callback: Optional[Callable] = None, callback_steps: int = 1,
-            negative_time_ids: Optional[torch.Tensor] = None) -> torch.Tensor:
+            negative_time_ids: Optional[torch.Tensor] = None, count_from_start: bool = False) -> torch.Tensor:
         """latents [n,4,h,w] (already scaled by init_noise_sigma; host or device); embeds host or device tensors.
         Returns the latents after the last executed step as a new device tensor.
 
@@ -100,7 +100,12 @@ class DenoiseEngine:
         are the output of a `stop_after=k` call with the same schedule (two-phase PNS: preview all candidates,
         continue only the winner).  `num_loop_steps` = k truncates the timestep list to its first k entries the way
         `denoising_end` does (custom_pipelines.py:307-316: the gating fractions of :326 then use k, the sigma table
-        stays the full schedule's).  `guidance_scale <= 1` runs the UNet on the positive branch only (:223)."""
+        stays the full schedule's).  `guidance_scale <= 1` runs the UNet on the positive branch only (:223).
+
+        `count_from_start=True` is img2img (`start_step` = t_start of `strength`, the latents noised to sigma[t_start]):
+        the control_guidance_start/end fractions and the callback's step index then count the executed steps from 0 over
+        the truncated list (steps start_step .. loop end), as `enumerate(timesteps)` does in [3P] diffusers' img2img
+        loop.  The default counts from the start of the full schedule (a resumed PNS trajectory)."""
         use_cfg = guidance_scale > 1.0                                            # :223
         if use_cfg and (negative_prompt_embeds is None or negative_pooled is None):
             raise IHError("classifier-free guidance needs negative_prompt_embeds / negative_pooled")
@@ -134,9 +139,12 @@ class DenoiseEngine:
         ops.scale_model_input(st["latents"], st["model_in"], sigmas, st["step"], duplicate=use_cfg)   # :332-334
 
         steps = loop_T if stop_after is None else min(stop_after, loop_T)
+        origin = start_step if count_from_start else 0                            # index of the first counted step
+        n_counted = loop_T - origin
 
         def scale_at(i: int) -> float:
-            off = (i / loop_T < control_guidance_start) or ((i + 1) / loop_T > control_guidance_end)   # :326-329
+            j = i - origin
+            off = (j / n_counted < control_guidance_start) or ((j + 1) / n_counted > control_guidance_end)   # :326-329
             return 0.0 if off else float(ip_scale)
 
         def gkey(scale: float):
@@ -172,8 +180,8 @@ class DenoiseEngine:
             else:
                 self.set_scale(sc)
                 self._step(st, timesteps, sigmas, guidance_scale, use_cfg, rescale)
-            if callback is not None and i % callback_steps == 0:                  # :359-363 (Euler: order 1, no warm-up)
-                callback(i, timesteps[i], st["latents"])
+            if callback is not None and (i - origin) % callback_steps == 0:       # :359-363 (Euler: order 1, no warm-up)
+                callback(i - origin, timesteps[i], st["latents"])
         self.set_scale(ip_scale)
         return st["latents"].clone()
 

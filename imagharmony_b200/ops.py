@@ -176,6 +176,62 @@ def conv3x3(x: torch.Tensor, w_packed: torch.Tensor, bias: Optional[torch.Tensor
     return out
 
 
+def conv3x3_s2_padbr(x: torch.Tensor, w_packed: torch.Tensor, bias: Optional[torch.Tensor] = None, *,
+                     out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """conv3x3(F.pad(x, (0, 1, 0, 1)), stride=2) + bias: the VAE encoder's Downsample2D(padding=0).  x NHWC [B,H,W,Cin]
+    (H, W even), w_packed [Cout, 9*Cin] (pack_conv3x3_weight); returns [B, H/2, W/2, Cout]."""
+    lib = _lib.load()
+    _req(x, "x"); _req(w_packed, "w")
+    B, H, W, Cin = x.shape
+    Cout = w_packed.shape[0]
+    if not x.is_contiguous() or not w_packed.is_contiguous() or w_packed.shape[1] != 9 * Cin:
+        raise IHError("conv3x3_s2_padbr: x must be contiguous NHWC and w_packed [Cout, 9*Cin]")
+    if out is None:
+        out = torch.empty((B, H // 2, W // 2, Cout), dtype=torch.float16, device=x.device)
+    check(lib.ih_conv2d_s2_padbr_f16(x.data_ptr(), w_packed.data_ptr(), _p(bias), out.data_ptr(), B, H, W, Cin, Cout,
+                                     _stream()), "ih_conv2d_s2_padbr_f16")
+    return out
+
+
+def image_im2col3x3(rgb_u8: torch.Tensor, kpad: int = 32, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """uint8 RGB NHWC [B, H, W, 3] -> A [B*H*W, kpad] of the normalised image 2 * (v / 255) - 1 (k = ci*9 + ky*3 + kx,
+    zero padded): the VAE encoder's conv_in as a tensor-core GEMM straight from the PIL pixels."""
+    lib = _lib.load()
+    _req(rgb_u8, "rgb_u8", torch.uint8)
+    B, H, W, C = rgb_u8.shape
+    if C != 3 or not rgb_u8.is_contiguous():
+        raise IHError("image_im2col3x3: contiguous uint8 RGB NHWC [B, H, W, 3] required")
+    if out is None:
+        out = torch.empty((B * H * W, kpad), dtype=torch.float16, device=rgb_u8.device)
+    check(lib.ih_image_im2col3x3_u8(rgb_u8.data_ptr(), out.data_ptr(), B, H, W, kpad, _stream()), "ih_image_im2col3x3_u8")
+    return out
+
+
+def vae_sample_add_noise(moments: torch.Tensor, eps: Optional[torch.Tensor], noise: torch.Tensor, channels: int,
+                         scaling_factor: float, sigma: float, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """img2img initial latents: moments NHWC [Bm, h, w, ldm] (mean, logvar), eps fp32 NCHW [Be, C, h, w] (None: the
+    moments' first C channels are the latents), noise fp16 NCHW [B, C, h, w] -> NCHW fp16
+    fp16(fp16(sf * fp16(mean + std * eps)) + fp16(noise * fp16(sigma))); image b uses moments b % Bm, eps b % Be."""
+    lib = _lib.load()
+    _req(moments, "moments"); _req(noise, "noise")
+    Bm, h, w, ldm = moments.shape
+    B = noise.shape[0]
+    if not moments.is_contiguous() or not noise.is_contiguous() or tuple(noise.shape) != (B, channels, h, w):
+        raise IHError(f"vae_sample_add_noise: contiguous moments and noise [B, {channels}, {h}, {w}] required")
+    Be = 0
+    if eps is not None:
+        _req(eps, "eps", torch.float32)
+        Be = eps.shape[0]
+        if not eps.is_contiguous() or tuple(eps.shape[1:]) != (channels, h, w):
+            raise IHError(f"vae_sample_add_noise: eps must be contiguous [Be, {channels}, {h}, {w}]")
+    if out is None:
+        out = torch.empty((B, channels, h, w), dtype=torch.float16, device=moments.device)
+    check(lib.ih_vae_sample_add_noise_f16(moments.data_ptr(), ldm, Bm, _p(eps), Be, noise.data_ptr(), out.data_ptr(), B,
+                                          channels, h, w, float(scaling_factor), float(sigma), _stream()),
+          "ih_vae_sample_add_noise_f16")
+    return out
+
+
 def pack_conv3x3_weight(w_oihw: torch.Tensor) -> torch.Tensor:
     """[Cout, Cin, 3, 3] (nn.Conv2d) -> [Cout, 9*Cin] tap-major, the layout ih_conv2d_f16 expects."""
     Cout, Cin, kh, kw = w_oihw.shape

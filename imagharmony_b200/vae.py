@@ -1,8 +1,10 @@
-"""Native SDXL VAE decoder (scope row f1: custom_pipelines.py:365-386 `vae.decode(latents / scaling_factor)` + postprocess).
+"""Native SDXL VAE decoder (scope row f1: custom_pipelines.py:365-386 `vae.decode(latents / scaling_factor)` + postprocess)
+and encoder (row f5, image-to-image editing: `AutoencoderKLEncoder`, see its docstring).
 
-Module tree and state-dict keys are those of [3P] diffusers==0.30.0 `AutoencoderKL` (`post_quant_conv.*`, `decoder.*`;
-encoder / quant_conv keys of a full checkpoint are ignored), so `vae/diffusion_pytorch_model.safetensors` loads without
-a key map.  Every operator runs on the sm_100a kernels of this package:
+Module tree and state-dict keys are those of [3P] diffusers==0.30.0 `AutoencoderKL` (decoder: `post_quant_conv.*`,
+`decoder.*`; encoder: `encoder.*`, `quant_conv.*`; each half ignores the other's keys), so
+`vae/diffusion_pytorch_model.safetensors` loads without a key map.  Every operator of the decoder runs on the sm_100a
+kernels of this package:
 
 * `post_quant_conv` (1x1, 4->4), the division by `scaling_factor` and `decoder.conv_in` (3x3, 4->C) are ONE tensor-core
   GEMM: the latent gets a constant-one fifth channel, `ih_im2col3x3_nchw_f16` builds the [B*h*w, 45 -> 64] patch matrix
@@ -325,6 +327,206 @@ class AutoencoderKLDecoder(nn.Module):
         x = ops.groupnorm(x, dec.conv_norm_out.weight, dec.conv_norm_out.bias, groups=g, eps=1e-6 * s * s, silu=True)
         x = ops.conv3x3(x, self._w_out, self._b_out)
         return ops.nhwc_to_nchw(x, self.config.out_channels)
+
+
+class VAEDownsample(nn.Module):
+    """diffusers Downsample2D(padding=0): conv3x3(F.pad(x, (0, 1, 0, 1)), stride 2) as one ih_conv2d_s2_padbr_f16."""
+
+    def __init__(self, ch: int):
+        super().__init__()
+        self.conv = nn.Conv2d(ch, ch, 3, stride=2, padding=0)
+        self._w = None
+
+    def finalize(self, s: float = 1.0):
+        self._w = ops.pack_conv3x3_weight(self.conv.weight.detach())
+        self._b = _scaled(self.conv.bias, s)
+
+    def forward(self, x):
+        return ops.conv3x3_s2_padbr(x, self._w, self._b)     # linear in the scaled stream: only the bias scales
+
+
+class VAEDownBlock(nn.Module):
+    def __init__(self, cin: int, cout: int, n_res: int, groups: int, add_down: bool):
+        super().__init__()
+        self.resnets = nn.ModuleList([VAEResnetBlock(cin if j == 0 else cout, cout, groups) for j in range(n_res)])
+        if add_down:
+            self.downsamplers = nn.ModuleList([VAEDownsample(cout)])
+        self.has_down = add_down
+
+    def forward(self, x):
+        for r in self.resnets:
+            x = r(x)
+        return self.downsamplers[0](x) if self.has_down else x
+
+
+class Encoder(nn.Module):
+    def __init__(self, cfg: VAEConfig):
+        super().__init__()
+        ch = cfg.block_out_channels
+        g = cfg.norm_num_groups
+        self.conv_in = nn.Conv2d(cfg.in_channels, ch[0], 3, padding=1)
+        downs: List[nn.Module] = []
+        prev = ch[0]
+        for i, c in enumerate(ch):
+            downs.append(VAEDownBlock(prev, c, cfg.layers_per_block, g, add_down=i < len(ch) - 1))
+            prev = c
+        self.down_blocks = nn.ModuleList(downs)
+        self.mid_block = VAEMidBlock(ch[-1], g)
+        self.conv_norm_out = nn.GroupNorm(g, ch[-1], eps=1e-6)
+        self.conv_out = nn.Conv2d(ch[-1], 2 * cfg.latent_channels, 3, padding=1)
+
+
+class AutoencoderKLEncoder(nn.Module):
+    """`encode(image)` = the moments of diffusers `vae.encode(image).latent_dist` (mean, logvar); the posterior sample,
+    `scaling_factor` and the scheduler's `add_noise` follow in one kernel (`ops.vae_sample_add_noise`).
+
+    * conv_in (3 -> C) is a GEMM over the im2col rows of the image: straight from the uint8 PIL pixels
+      (`ih_image_im2col3x3_u8`, which also normalises 2 v / 255 - 1) or from a float NCHW tensor in [-1, 1]
+      (`ih_im2col3x3_nchw_f16`);
+    * down blocks of ResnetBlock2D (the decoder's VAEResnetBlock) and Downsample2D(padding=0) (`ih_conv2d_s2_padbr_f16`),
+      the decoder's mid block (resnet, attention, resnet);
+    * GroupNorm + SiLU, then conv_out with quant_conv folded in: W' = Wq Wco, b' = Wq bco + bq (exact in real
+      arithmetic), Cout padded 8 -> 16.  The moments come out as NHWC [B, h, w, 16], channels [0, L) mean,
+      [L, 2L) logvar.
+
+    The residual stream is scaled by `stream_scale` exactly as in the decoder (module docstring); conv_out reads the
+    GroupNorm output, so the moments are at scale 1."""
+
+    def __init__(self, cfg: VAEConfig = SDXL_VAE):
+        super().__init__()
+        self.config = cfg
+        self.encoder = Encoder(cfg)
+        self.quant_conv = nn.Conv2d(2 * cfg.latent_channels, 2 * cfg.latent_channels, 1)
+        self._w_in = self._w_out = self._b_out = None
+        self.use_tiling = False             # pipeline.enable_vae_tiling() (test.py:73)
+        self.stream_scale = 2.0 ** -7 if getattr(cfg, "force_upcast", True) else 1.0
+
+    KPAD_IN = 32                            # conv_in: 3 * 9 = 27 im2col columns padded to a multiple of 8
+    COUT_PAD = 16                           # conv_out: 2 L = 8 moment channels padded to 16
+
+    @classmethod
+    def from_state_dict(cls, cfg: VAEConfig, sd: Dict[str, torch.Tensor], device="cuda",
+                        stream_scale: Optional[float] = None) -> "AutoencoderKLEncoder":
+        """Loads the `encoder.*` / `quant_conv.*` keys of a diffusers AutoencoderKL state dict (other keys ignored)."""
+        with torch.device("meta"):
+            m = cls(cfg)
+        if stream_scale is not None:
+            if stream_scale <= 0 or math.log2(stream_scale) != int(math.log2(stream_scale)):
+                raise IHError("stream_scale must be a power of two")
+            m.stream_scale = float(stream_scale)
+        m = m.to_empty(device=device)
+        own = m.state_dict()
+        missing = [k for k in own if k not in sd]
+        if missing:
+            raise KeyError(f"VAE checkpoint lacks {len(missing)} encoder keys, e.g. {missing[:3]}")
+        m.load_state_dict({k: sd[k].to(device=device, dtype=torch.float16).reshape(own[k].shape) for k in own})
+        m = m.half().eval()
+        m.finalize()
+        return m
+
+    def finalize(self) -> None:
+        s = self.stream_scale
+        for mod in self.modules():
+            if isinstance(mod, (VAEResnetBlock, VAEAttention, VAEDownsample)):
+                mod.finalize(s)
+        enc = self.encoder
+        dt = enc.conv_in.weight.dtype
+        w_in = enc.conv_in.weight.detach()
+        C0 = w_in.shape[0]
+        w = torch.zeros((C0, self.KPAD_IN), dtype=dt, device=w_in.device)
+        w[:, :w_in[0].numel()] = w_in.reshape(C0, -1)                                 # k = ci*9 + ky*3 + kx
+        self._w_in = w.contiguous()
+        self._b_in = _scaled(enc.conv_in.bias, s)
+        L2 = 2 * self.config.latent_channels
+        wq = self.quant_conv.weight.detach().float().reshape(L2, L2)                    # [o, m]
+        wco = enc.conv_out.weight.detach().float()                                     # [m, C, 3, 3]
+        folded_w = torch.einsum("om,mcyx->ocyx", wq, wco)
+        folded_b = wq @ enc.conv_out.bias.detach().float() + self.quant_conv.bias.detach().float()
+        w_out = torch.zeros((self.COUT_PAD,) + tuple(wco.shape[1:]), dtype=dt, device=wco.device)
+        w_out[:L2] = folded_w.to(dt)
+        self._w_out = ops.pack_conv3x3_weight(w_out)
+        b_out = torch.zeros((self.COUT_PAD,), dtype=dt, device=wco.device)
+        b_out[:L2] = folded_b.to(dt)
+        self._b_out = b_out
+
+    # ---- forward -----------------------------------------------------------------------------------------------
+    @torch.no_grad()
+    def encode(self, image: torch.Tensor) -> torch.Tensor:
+        """image: uint8 RGB NHWC [B, H, W, 3] (PIL pixels) or float NCHW [B, 3, H, W] in [-1, 1]; H, W multiples of 8.
+        Returns the moments NHWC [B, H/8, W/8, 16] (fp16; channels [0, L) mean, [L, 2L) logvar, the rest zero).
+        With `use_tiling` and an image larger than one tile (`sample_size` pixels) the image is encoded tile by tile and
+        the moments are blended, [3P] diffusers `AutoencoderKL.tiled_encode`."""
+        if self._w_in is None:
+            raise IHError("AutoencoderKLEncoder.finalize() has not run (use from_state_dict)")
+        nhwc = image.dtype == torch.uint8
+        H, W = (image.shape[1], image.shape[2]) if nhwc else (image.shape[2], image.shape[3])
+        if H % 8 or W % 8:
+            raise IHError(f"VAE encoder: image size {H}x{W} is not a multiple of 8")
+        t = self.config.sample_size
+        if self.use_tiling and (H > t or W > t):
+            return self._tiled_encode(image, nhwc)
+        return self._encode_tile(image, nhwc)
+
+    def _tiled_encode(self, x: torch.Tensor, nhwc: bool) -> torch.Tensor:
+        """[3P] tiled_encode: tiles of `sample_size` pixels every (1 - overlap) tile, each encoded on its own, the moments
+        cross-faded over `tile_latent_min_size * overlap` latents with the tile above and the tile to the left and
+        cropped to the rest of the latent tile.  The cross-fade is elementwise torch glue (NHWC moments)."""
+        cfg = self.config
+        ts = cfg.sample_size
+        stride = int(ts * (1 - cfg.tile_overlap_factor))
+        blend = int(cfg.tile_latent_min_size * cfg.tile_overlap_factor)
+        limit = cfg.tile_latent_min_size - blend
+        H, W = (x.shape[1], x.shape[2]) if nhwc else (x.shape[2], x.shape[3])
+        rows = []
+        for i in range(0, H, stride):
+            row = []
+            for j in range(0, W, stride):
+                tile = x[:, i:i + ts, j:j + ts, :] if nhwc else x[:, :, i:i + ts, j:j + ts]
+                row.append(self._encode_tile(tile.contiguous(), nhwc).float())
+            rows.append(row)
+
+        def blend_v(a, b, ext):
+            ext = min(a.shape[1], b.shape[1], ext)
+            wgt = (torch.arange(ext, device=b.device, dtype=torch.float32) / ext).view(1, ext, 1, 1)
+            b[:, :ext] = a[:, -ext:] * (1 - wgt) + b[:, :ext] * wgt
+            return b
+
+        def blend_h(a, b, ext):
+            ext = min(a.shape[2], b.shape[2], ext)
+            wgt = (torch.arange(ext, device=b.device, dtype=torch.float32) / ext).view(1, 1, ext, 1)
+            b[:, :, :ext] = a[:, :, -ext:] * (1 - wgt) + b[:, :, :ext] * wgt
+            return b
+
+        out_rows = []
+        for i, row in enumerate(rows):
+            out_row = []
+            for j, tile in enumerate(row):
+                if i > 0:
+                    tile = blend_v(rows[i - 1][j], tile, blend)
+                if j > 0:
+                    tile = blend_h(row[j - 1], tile, blend)
+                out_row.append(tile[:, :limit, :limit])
+            out_rows.append(torch.cat(out_row, dim=2))
+        return torch.cat(out_rows, dim=1).to(self._w_in.dtype).contiguous()
+
+    def _encode_tile(self, x: torch.Tensor, nhwc: bool) -> torch.Tensor:
+        enc = self.encoder
+        dt = self._w_in.dtype                                     # fp16 on the GPU (fp32 only in the CPU wiring test)
+        if nhwc:
+            B, H, W, _ = x.shape
+            a = ops.image_im2col3x3(x, self.KPAD_IN)
+        else:
+            B, _, H, W = x.shape
+            a = ops.im2col3x3_nchw(x.to(dt).contiguous(), self.KPAD_IN)
+        s = self.stream_scale
+        h = ops.linear(a, self._w_in, self._b_in, alpha=s).reshape(B, H, W, -1)       # s * conv_in(image)
+        for blk in enc.down_blocks:
+            h = blk(h)
+        h = enc.mid_block(h)
+        g = self.config.norm_num_groups
+        h = ops.groupnorm(h, enc.conv_norm_out.weight, enc.conv_norm_out.bias, groups=g, eps=1e-6 * s * s, silu=True)
+        return ops.conv3x3(h, self._w_out, self._b_out)                               # quant_conv(conv_out(.)), scale 1
+
 
 
 def postprocess(image: torch.Tensor, output_type: str = "pil"):

@@ -89,6 +89,13 @@ int ih_conv2d_shortcut_f16(const void* x, const void* w, const void* bias, const
 int ih_conv2d_scaled_f16(const void* x, const void* w, const void* bias, const void* residual, void* out, int B, int Hin,
                          int Win, int Cin, int Cout, int stride, float alpha, void* stream);
 
+/* 3x3 conv, stride 2, padding on the bottom and right only: conv(F.pad(x, (0, 1, 0, 1)), stride=2), input row
+ * 2*oy + dy (the other stride-2 convs read 2*oy + dy - 1).  Replaces the VAE encoder's Downsample2D(padding=0)
+ * ([3P] diffusers AutoencoderKL.encode, img2img).  Weight layout as ih_conv2d_f16; even H, W; Cin % 64 == 0.
+ * out = conv(x) + bias: linear in the scaled residual stream, so the caller scales only the bias. */
+int ih_conv2d_s2_padbr_f16(const void* x, const void* w, const void* bias, void* out, int B, int Hin, int Win, int Cin,
+                           int Cout, void* stream);
+
 /* Multi-head attention, head_dim 64, softmax scale 1/8, no mask.
  *   q: [B, Nq, *] rows with ldq elements per row, head h at columns [h*64, h*64+64) (same for k, v, out).
  *   Self attention (n_ip == 0): out = softmax(q k^T / 8) v over Nk keys.
@@ -187,6 +194,19 @@ int ih_conv_out_f16(const void* x, const void* w, const void* bias, void* out_nc
 /* conv_in on the tensor-core GEMM: im2col of the NCHW latent into A [B*H*W, Kpad] (k = ci*9 + ky*3 + kx, zero padded),
  * to be multiplied with the OIHW weight flattened (and zero padded) to [Cout, Kpad] by ih_gemm_f16. */
 int ih_im2col3x3_nchw_f16(const void* x_nchw, void* out, int B, int Cin, int H, int W, int Kpad, void* stream);
+/* VAE encoder conv_in on the tensor-core GEMM, straight from the PIL pixels: uint8 RGB NHWC [B,H,W,3] -> im2col rows
+ * [B*H*W, Kpad] (k = ci*9 + ky*3 + kx, zero padding 1, K padding zero) of fp16(2 * (v / 255) - 1), the fp32 rounding
+ * points of [3P] diffusers VaeImageProcessor (pil_to_numpy, normalize).  Kpad % 8 == 0, Kpad >= 27. */
+int ih_image_im2col3x3_u8(const void* rgb_u8, void* out, int B, int H, int W, int Kpad, void* stream);
+/* img2img initial latents from the encoder's moments (NHWC [Bm, h, w, ldm]: mean in channels [0, C), logvar in [C, 2C)):
+ *   z = fp16(sf * fp16(mean + exp(0.5 clamp(logvar, -30, 20)) * eps))   ([3P] DiagonalGaussianDistribution.sample in fp32,
+ *       cast, `scaling_factor * latents` in fp16);  eps == NULL: z = mean (latents passed as they are, Be ignored);
+ *   out = fp16(z + fp16(noise * fp16(sigma)))   ([3P] EulerDiscreteScheduler.add_noise on fp16 tensors).
+ * eps fp32 NCHW [Be, C, h, w], noise fp16 NCHW [B, C, h, w], out fp16 NCHW [B, C, h, w]; output image b reads moments
+ * b % Bm and eps b % Be. */
+int ih_vae_sample_add_noise_f16(const void* moments, long long ldm, int Bm, const void* eps_f32, int Be, const void* noise,
+                                void* out_nchw, int B, int C, int h, int w, float scaling_factor, float sigma,
+                                void* stream);
 /* conv_out on ih_conv2d_f16 with Cout padded to 16: gather NHWC [B, HW, ldc] channels [0, C) into NCHW [B, C, HW]. */
 int ih_nhwc_to_nchw_f16(const void* x, long long ldc, void* out, int B, long long HW, int C, void* stream);
 

@@ -266,3 +266,216 @@ class StableDiffusionXLCustomPipeline:
         if not return_dict:
             return (image,)
         return StableDiffusionXLPipelineOutput(images=image)
+
+
+class StableDiffusionXLImg2ImgCustomPipeline(StableDiffusionXLCustomPipeline):
+    """Image-to-image editing on the same call surface: `image=` (the source) and `strength=` on top of the
+    text-to-image parameters, following [3P] diffusers==0.30.0 `StableDiffusionXLImg2ImgPipeline`.
+
+    The source image is encoded by the native VAE encoder (`imagharmony_b200.vae.AutoencoderKLEncoder`), its posterior
+    sample is scaled and noised to sigma[t_start] in one kernel, and the denoise loop runs only the last
+    T - t_start = min(int(T * strength), T) steps of the T-step schedule.  IPAdapterXL.generate(image=..., strength=...)
+    reaches this call through its **kwargs."""
+
+    def __init__(self, unet: UNet2DConditionModel, prompt_encoder: Optional[Callable] = None,
+                 vae_decode: Optional[Callable] = None, scheduler: Optional[EulerDiscreteScheduler] = None,
+                 vae=None, vae_encoder=None):
+        super().__init__(unet, prompt_encoder=prompt_encoder, vae_decode=vae_decode, scheduler=scheduler, vae=vae)
+        self.vae_encoder = vae_encoder      # imagharmony_b200.vae.AutoencoderKLEncoder or None
+
+    # ---- construction ------------------------------------------------------------------------------------------
+    @classmethod
+    def from_random(cls, cfg: UNetConfig = SDXL_BASE, seed: int = 0, device="cuda", vae_cfg=None):
+        """As the text-to-image pipeline, plus a random-init VAE encoder when `vae_cfg` is given."""
+        pipe = super().from_random(cfg, seed=seed, device=device, vae_cfg=vae_cfg)
+        if vae_cfg is not None:
+            from imagharmony_b200.vae import AutoencoderKLEncoder
+            from imagharmony_b200.weights import random_state_dict, shapes_of
+            with torch.device("meta"):
+                eshapes = shapes_of(AutoencoderKLEncoder(vae_cfg))
+            gen_dev = device if str(device).startswith("cuda") else "cpu"
+            pipe.vae_encoder = AutoencoderKLEncoder.from_state_dict(
+                vae_cfg, random_state_dict(eshapes, seed + 18, device=gen_dev), device=device)
+        return pipe
+
+    @classmethod
+    def from_pretrained(cls, path: str, torch_dtype=torch.float16, add_watermarker: bool = False, device="cuda",
+                        cfg: UNetConfig = SDXL_BASE, vae_cfg=None, **kwargs):
+        """As the text-to-image pipeline; the encoder half is loaded from the same `vae/` safetensors, with the same
+        `force_upcast` / `scaling_factor` from its config.json."""
+        pipe = super().from_pretrained(path, torch_dtype=torch_dtype, add_watermarker=add_watermarker, device=device,
+                                       cfg=cfg, vae_cfg=vae_cfg, **kwargs)
+        if pipe.vae is not None:
+            from safetensors.torch import load_file
+            from imagharmony_b200.vae import AutoencoderKLEncoder
+            for name in ("diffusion_pytorch_model.fp16.safetensors", "diffusion_pytorch_model.safetensors"):
+                vf = os.path.join(path, "vae", name)
+                if os.path.exists(vf):
+                    pipe.vae_encoder = AutoencoderKLEncoder.from_state_dict(pipe.vae.config, load_file(vf), device=device)
+                    break
+        return pipe
+
+    def enable_vae_tiling(self):  # test.py:73; tiles both halves
+        super().enable_vae_tiling()
+        if self.vae_encoder is not None:
+            self.vae_encoder.use_tiling = True
+
+    # ---- img2img -----------------------------------------------------------------------------------------------
+    @staticmethod
+    def get_timesteps(num_inference_steps: int, strength: float) -> Tuple[int, int]:
+        """[3P] get_timesteps: -> (t_start, executed steps), init_timestep = min(int(T * strength), T)."""
+        init_timestep = min(int(num_inference_steps * strength), num_inference_steps)
+        t_start = max(num_inference_steps - init_timestep, 0)
+        return t_start, num_inference_steps - t_start
+
+    def preprocess_image(self, image):
+        """-> ("pixels", uint8 NHWC [B, H, W, 3]) for PIL input (size rounded down to a multiple of 8 with a Lanczos resize,
+        [3P] VaeImageProcessor), ("image", float32 NCHW in [-1, 1]) for a 3-channel tensor (normalised 2 x - 1 unless its
+        minimum is < 0), ("latents", fp16 NCHW) for a tensor with latent_channels channels (used as it is)."""
+        import numpy as np
+        from PIL import Image
+        if isinstance(image, Image.Image) or (isinstance(image, (list, tuple)) and image
+                                              and isinstance(image[0], Image.Image)):
+            images = [image] if isinstance(image, Image.Image) else list(image)
+            arrs = []
+            for im in images:
+                im = im.convert("RGB")
+                w, h = (im.width // self.vae_scale_factor) * self.vae_scale_factor, \
+                       (im.height // self.vae_scale_factor) * self.vae_scale_factor
+                if (w, h) != im.size:
+                    im = im.resize((w, h), resample=Image.LANCZOS)
+                arrs.append(np.asarray(im, dtype=np.uint8))
+            if len({a.shape for a in arrs}) != 1:
+                raise ValueError("all source images must have the same size")
+            return "pixels", torch.from_numpy(np.stack(arrs)).to(self.device)
+        if isinstance(image, torch.Tensor):
+            x = image if image.dim() == 4 else image.unsqueeze(0)
+            if x.shape[1] == self.unet.config.in_channels:
+                return "latents", x.to(self.device, torch.float16).contiguous()
+            x = x.to(torch.float32)
+            if x.min() >= 0:
+                x = 2.0 * x - 1.0
+            return "image", x.to(self.device).contiguous()
+        raise TypeError(f"image must be a PIL image, a list of PIL images or a torch tensor, got {type(image)}")
+
+    def prepare_img2img_latents(self, image, batch: int, generator, sigma: float) -> Tuple[torch.Tensor, Tuple[int, int]]:
+        """Initial latents [batch, 4, h, w] fp16 on the device, and the source image size (H, W).
+
+        Draw order ([3P] prepare_latents + retrieve_latents + randn_tensor): the posterior eps (fp32, the mean's shape)
+        first, then the noise (fp16).  With a generator list, one [1, 4, h, w] eps per batch slot (the images replicated
+        to the batch) and then one noise per slot, so a candidate does not depend on its batch slot."""
+        kind, x = self.preprocess_image(image)
+        n_img = x.shape[0]
+        if batch % n_img:
+            raise ValueError(f"cannot duplicate {n_img} source images to a batch of {batch}")
+        if isinstance(generator, list) and len(generator) != batch:
+            raise ValueError(f"got {len(generator)} generators for a batch of {batch}")
+        L = self.unet.config.in_channels
+
+        def randn(shape, g, dtype):
+            return torch.randn(shape, generator=g, device=g.device if g is not None else "cpu", dtype=dtype)
+        if kind == "latents":
+            moments, eps = x.permute(0, 2, 3, 1).contiguous(), None
+            h, w = x.shape[2], x.shape[3]
+            size = (h * self.vae_scale_factor, w * self.vae_scale_factor)
+        else:
+            if self.vae_encoder is None:
+                raise IHError("this pipeline has no VAE encoder: build it with from_random(vae_cfg=...) or from_pretrained "
+                              "with a vae/ folder, or pass latents as a 4-channel image tensor")
+            size = (x.shape[1], x.shape[2]) if kind == "pixels" else (x.shape[2], x.shape[3])
+            moments = self.vae_encoder.encode(x)                  # once per source image: the moments are deterministic
+            h, w = moments.shape[1], moments.shape[2]
+            if isinstance(generator, list):
+                eps = torch.cat([randn((1, L, h, w), g, torch.float32).to(self.device) for g in generator], dim=0)
+            else:
+                eps = randn((n_img, L, h, w), generator, torch.float32).to(self.device)
+        if isinstance(generator, list):
+            noise = torch.cat([randn((1, L, h, w), g, torch.float16).to(self.device) for g in generator], dim=0)
+        else:
+            noise = randn((batch, L, h, w), generator, torch.float16).to(self.device)
+        from imagharmony_b200 import ops
+        sf = 1.0 if eps is None else self.vae_encoder.config.scaling_factor
+        return ops.vae_sample_add_noise(moments, eps, noise, L, sf, sigma), size
+
+    @torch.no_grad()
+    def __call__(self, prompt: Optional[Union[str, List[str]]] = None, prompt_2=None, image=None, strength: float = 0.3,
+                 height: Optional[int] = None, width: Optional[int] = None, num_inference_steps: int = 50,
+                 denoising_end: Optional[float] = None, guidance_scale: float = 5.0, negative_prompt=None,
+                 negative_prompt_2=None, num_images_per_prompt: Optional[int] = 1, eta: float = 0.0, generator=None,
+                 latents: Optional[torch.Tensor] = None, prompt_embeds: Optional[torch.Tensor] = None,
+                 negative_prompt_embeds: Optional[torch.Tensor] = None,
+                 pooled_prompt_embeds: Optional[torch.Tensor] = None,
+                 negative_pooled_prompt_embeds: Optional[torch.Tensor] = None, output_type: Optional[str] = "pil",
+                 return_dict: bool = True, callback=None, callback_steps: int = 1,
+                 cross_attention_kwargs: Optional[Dict[str, Any]] = None, guidance_rescale: float = 0.0,
+                 original_size: Optional[Tuple[int, int]] = None, crops_coords_top_left: Tuple[int, int] = (0, 0),
+                 target_size: Optional[Tuple[int, int]] = None, negative_original_size=None,
+                 negative_crops_coords_top_left=(0, 0), negative_target_size=None,
+                 control_guidance_start: float = 0.0, control_guidance_end: float = 1.0, aesthetic_score: float = 6.0,
+                 negative_aesthetic_score: float = 2.5, **ignored):
+        """The text-to-image parameters plus `image` and `strength`.  The latent size comes from the image (`height` /
+        `width` and `latents` are not used); `aesthetic_score*` are accepted and ignored (SDXL-base has
+        requires_aesthetics_score = false, so its time ids equal the text-to-image ones)."""
+        if image is None:
+            raise ValueError("img2img needs a source `image`")
+        if not 0.0 <= strength <= 1.0:
+            raise ValueError(f"The value of strength should be in [0.0, 1.0] but is {strength}")
+        if callback is not None and (not isinstance(callback_steps, int) or callback_steps <= 0):
+            raise ValueError(f"`callback_steps` has to be a positive integer but is {callback_steps}")
+        t_start, n_exec = self.get_timesteps(num_inference_steps, strength)
+        if n_exec < 1:
+            raise ValueError(f"strength {strength} with num_inference_steps {num_inference_steps} leaves no denoising "
+                             "step (the number of steps run is min(int(num_inference_steps * strength), num_inference_steps))")
+        do_classifier_free_guidance = guidance_scale > 1.0
+        (prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds, negative_pooled_prompt_embeds) = \
+            self.encode_prompt(prompt, prompt_2, None, num_images_per_prompt, do_classifier_free_guidance,
+                               negative_prompt, negative_prompt_2, prompt_embeds, negative_prompt_embeds,
+                               pooled_prompt_embeds, negative_pooled_prompt_embeds)
+        batch = prompt_embeds.shape[0]
+        self.scheduler.set_timesteps(num_inference_steps)
+        sigma = float(self.scheduler.sigmas[t_start])                   # add_noise at the begin index t_start
+        lat, size = self.prepare_img2img_latents(image, batch, generator, sigma)
+        original_size = original_size or size
+        target_size = target_size or size
+
+        def time_ids(size, crop, target):
+            return torch.tensor([list(size) + list(crop) + list(target)], dtype=torch.float32).repeat(batch, 1)
+        add_time_ids = time_ids(original_size, crops_coords_top_left, target_size)
+        negative_add_time_ids = None
+        if negative_original_size is not None and negative_target_size is not None:
+            negative_add_time_ids = time_ids(negative_original_size, negative_crops_coords_top_left, negative_target_size)
+        loop_steps = num_inference_steps                                # denoising_end cuts the full schedule's list
+        if denoising_end is not None and isinstance(denoising_end, float) and 0 < denoising_end < 1:
+            n_train = self.scheduler.num_train_timesteps
+            cutoff = int(round(n_train - denoising_end * n_train))
+            loop_steps = int(sum(1 for t in self.scheduler.timesteps if t >= cutoff))
+        conditioning_scale = 1.0
+        for attn_processor in self.unet.attn_processors.values():
+            if isinstance(attn_processor, IPAttnProcessor):
+                conditioning_scale = attn_processor.scale
+                break
+        if loop_steps > t_start:
+            out = self.engine.run(lat, prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds,
+                                  negative_pooled_prompt_embeds, add_time_ids, num_inference_steps,
+                                  guidance_scale=guidance_scale, ip_scale=conditioning_scale,
+                                  control_guidance_start=control_guidance_start,
+                                  control_guidance_end=control_guidance_end, guidance_rescale=guidance_rescale,
+                                  start_step=t_start, num_loop_steps=loop_steps, callback=callback,
+                                  callback_steps=callback_steps, negative_time_ids=negative_add_time_ids,
+                                  count_from_start=True)
+        else:
+            out = lat
+        self.set_scale(conditioning_scale)
+        if output_type == "latent":
+            image = out
+        elif self.vae_decode is not None:
+            image = self.vae_decode(out / 0.13025, output_type)
+        elif self.vae is not None:
+            from imagharmony_b200.vae import postprocess
+            image = postprocess(self.vae.decode(out), output_type)
+        else:
+            raise IHError("this pipeline has no VAE decoder: call with output_type='latent', build it with a `vae` "
+                          "(from_random(vae_cfg=...), from_pretrained with a vae/ folder) or pass a vae_decode callable")
+        if not return_dict:
+            return (image,)
+        return StableDiffusionXLPipelineOutput(images=image)
