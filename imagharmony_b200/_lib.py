@@ -110,6 +110,9 @@ SIGNATURES = {
     "ih_image_im2col3x3_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "ih_vae_sample_add_noise_f16": (c_int, [c_void_p, c_longlong, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int,
                                             c_int, c_int, c_int, c_float, c_float, c_void_p]),
+    "ih_vae_sample_inpaint_f16": (c_int, [c_void_p, c_longlong, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p,
+                                          c_int, c_int, c_int, c_int, c_float, c_float, c_int, c_void_p]),
+    "ih_latent_mask_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "ih_nhwc_to_nchw_f16": (c_int, [c_void_p, c_longlong, c_void_p, c_int, c_longlong, c_int, c_void_p]),
     "ih_euler_cfg_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_longlong, c_int,
                                   c_void_p]),
@@ -120,6 +123,9 @@ SIGNATURES = {
                                        ctypes.POINTER(c_float), ctypes.POINTER(c_float), c_void_p]),
     "ih_euler_step_ex": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_float, c_longlong, c_int,
                                  c_int, c_void_p]),
+    "ih_euler_step_inpaint": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_float, c_longlong,
+                                      c_int, c_int, c_void_p, c_int, c_longlong, c_void_p, c_void_p, c_void_p,
+                                      c_void_p]),
     "ih_scale_model_input": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_void_p]),
     "ih_scale_model_input_ex": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_int, c_void_p]),
 }

@@ -231,18 +231,56 @@ __global__ void conv_out_kernel(const __half* __restrict__ x, const __half* __re
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// Inpainting blend, applied inside the Euler kernels (BLEND = true) after the update and before the next step's
+// model_in is formed ([3P] diffusers StableDiffusionXLInpaintPipeline, 4-channel UNet, fp16 tensors):
+//   proper = z0                                    on the last executed step (*last == step index),
+//          = fp16(z0 + fp16(noise * fp16(sigma_next)))   otherwise (add_noise at the next sigma);
+//   latents = fp16(fp16(fp16(1 - m) * proper) + fp16(m * latents)).
+// The last step takes z0 itself, not add_noise with sigma 0: z0 + fp16(noise * 0) turns z0 = -0 into +0.
+// mask: uint8 {0, 1} [Bm, hw]; latent image b uses mask b % Bm.  z0 / noise: fp16 NCHW, the latents' shape.
+// ---------------------------------------------------------------------------------------------------------------
+struct InpaintBlend {
+  const unsigned char* mask;
+  const __half* z0;
+  const __half* noise;
+  const int* last;
+  long long hw;
+  int Bm;
+};
+
+__device__ __forceinline__ __half inpaint_blend(const InpaintBlend& bl, long long idx, int img, long long e,
+                                                bool last, float sig16_next, __half xh) {
+  const float m = (float)bl.mask[(long long)(img % bl.Bm) * bl.hw + e % bl.hw];
+  const float z = __half2float(bl.z0[idx]);
+  const float proper =
+      last ? z : __half2float(__float2half_rn(__fadd_rn(z, __half2float(__float2half_rn(
+                                                              __fmul_rn(__half2float(bl.noise[idx]), sig16_next))))));
+  const float keep = __half2float(__float2half_rn(__fmul_rn(__fsub_rn(1.f, m), proper)));
+  const float gen = __half2float(__float2half_rn(__fmul_rn(m, __half2float(xh))));
+  return __float2half_rn(__fadd_rn(keep, gen));
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // CFG + Euler. Rounding points follow the reference's fp16 tensor arithmetic (custom_pipelines.py:348-350) and
 // diffusers' EulerDiscreteScheduler.step (fp32 inside, result cast back to fp16).
 // ---------------------------------------------------------------------------------------------------------------
+template <bool BLEND>
 __global__ void euler_cfg_kernel(const __half* __restrict__ noise, __half* __restrict__ latents,
                                  __half* __restrict__ model_in, const float* __restrict__ sigmas,
-                                 const int* __restrict__ step, float guidance, long long per_image, int n_images) {
+                                 const int* __restrict__ step, float guidance, long long per_image, int n_images,
+                                 InpaintBlend bl) {
   pdl_launch_dependents();
   pdl_wait();
   const int i = *step;
   const float sigma = sigmas[i], sigma_next = sigmas[i + 1];
   const float den_next = sqrtf(sigma_next * sigma_next + 1.f);
   const long long total = per_image * n_images;
+  bool last = false;
+  float sig16_next = 0.f;
+  if constexpr (BLEND) {
+    last = i == *bl.last;
+    sig16_next = __half2float(__float2half_rn(sigma_next));
+  }
   for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
     const float u = __half2float(noise[idx]);
@@ -256,7 +294,11 @@ __global__ void euler_cfg_kernel(const __half* __restrict__ noise, __half* __res
     const float x0 = x - __half2float(__float2half_rn(sigma * eps));
     const float deriv = (x - x0) / sigma;
     const float xn = x + deriv * (sigma_next - sigma);
-    const __half xh = __float2half_rn(xn);
+    __half xh = __float2half_rn(xn);
+    if constexpr (BLEND) {
+      const int img = (int)(idx / per_image);
+      xh = inpaint_blend(bl, idx, img, idx - (long long)img * per_image, last, sig16_next, xh);
+    }
     latents[idx] = xh;
     const __half mi = __float2half_rn(__half2float(xh) / den_next);
     model_in[idx] = mi;
@@ -269,11 +311,12 @@ __global__ void euler_cfg_kernel(const __half* __restrict__ noise, __half* __res
 // image: a first sweep forms the guided prediction and its statistics (double accumulators, fixed reduction order:
 // deterministic), a second sweep -- the image is L1/L2 resident -- applies rescale + Euler.  n_images blocks of
 // 1024 threads; a 4 x 128 x 128 latent is 64 elements per thread.
+template <bool BLEND>
 __global__ void __launch_bounds__(1024) euler_ex_kernel(const __half* __restrict__ noise, __half* __restrict__ latents,
                                                          __half* __restrict__ model_in,
                                                          const float* __restrict__ sigmas, const int* __restrict__ step,
                                                          float guidance, float rescale, long long per_image,
-                                                         int n_images, int cfg) {
+                                                         int n_images, int cfg, InpaintBlend bl) {
   pdl_launch_dependents();
   pdl_wait();
   const int img = blockIdx.x;
@@ -282,6 +325,12 @@ __global__ void __launch_bounds__(1024) euler_ex_kernel(const __half* __restrict
   const float den_next = sqrtf(sigma_next * sigma_next + 1.f);
   const long long total = per_image * n_images;
   const long long base = (long long)img * per_image;
+  bool last = false;
+  float sig16_next = 0.f;
+  if constexpr (BLEND) {
+    last = i == *bl.last;
+    sig16_next = __half2float(__float2half_rn(sigma_next));
+  }
   auto guided = [&](long long idx, float& c_out) -> float {
     if (!cfg) {
       c_out = __half2float(noise[idx]);
@@ -343,7 +392,8 @@ __global__ void __launch_bounds__(1024) euler_ex_kernel(const __half* __restrict
     const float x0 = x - __half2float(__float2half_rn(sigma * eps));
     const float deriv = (x - x0) / sigma;
     const float xn = x + deriv * (sigma_next - sigma);
-    const __half xh = __float2half_rn(xn);
+    __half xh = __float2half_rn(xn);
+    if constexpr (BLEND) xh = inpaint_blend(bl, idx, img, e, last, sig16_next, xh);
     latents[idx] = xh;
     const __half mi = __float2half_rn(__half2float(xh) / den_next);
     model_in[idx] = mi;
@@ -752,9 +802,13 @@ __global__ void image_im2col3x3_u8_kernel(const unsigned char* __restrict__ x, _
   }
 }
 
+// INPAINT = true also writes z to z0_out (the blend's clean latents, fp16-exact) and, with pure_noise, sets
+// out = fp16(noise * sigma) with sigma = init_noise_sigma unrounded (strength 1: `noise * init_noise_sigma`).
+template <bool INPAINT>
 __global__ void vae_sample_add_noise_kernel(const __half* __restrict__ moments, long long ldm, int Bm,
                                             const float* __restrict__ eps, int Be, const __half* __restrict__ noise,
-                                            __half* __restrict__ out, int B, int C, long long HW, float sf, float sigma) {
+                                            __half* __restrict__ out, int B, int C, long long HW, float sf, float sigma,
+                                            __half* __restrict__ z0_out, int pure_noise) {
   pdl_launch_dependents();
   pdl_wait();
   const float sig16 = __half2float(__float2half_rn(sigma));
@@ -774,8 +828,32 @@ __global__ void vae_sample_add_noise_kernel(const __half* __restrict__ moments, 
     } else {
       z = __half2float(m[c]);                        // latents given as they are (4-channel image input)
     }
+    if constexpr (INPAINT) {
+      z0_out[i] = __float2half_rn(z);
+      if (pure_noise) {
+        out[i] = __float2half_rn(__fmul_rn(__half2float(noise[i]), sigma));
+        continue;
+      }
+    }
     const float ns = __half2float(__float2half_rn(__fmul_rn(__half2float(noise[i]), sig16)));
     out[i] = __float2half_rn(__fadd_rn(z, ns));
+  }
+}
+
+// Inpainting latent mask: uint8 grayscale [Bm, H, W] -> uint8 {0, 1} [Bm, H/8, W/8].  [3P] diffusers binarizes
+// v / 255 at 0.5 (v >= 128 for uint8 pixels) and takes the latent mask with F.interpolate's default nearest mode, so
+// latent (y, x) reads pixel (8y, 8x).
+__global__ void latent_mask_u8_kernel(const unsigned char* __restrict__ mask, unsigned char* __restrict__ out, int Bm,
+                                      int H, int W) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const int h = H / 8, w = W / 8;
+  const long long total = (long long)Bm * h * w;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int x = (int)(i % w);
+    const int y = (int)((i / w) % h);
+    const int b = (int)(i / ((long long)w * h));
+    out[i] = mask[((long long)b * H + 8 * y) * W + 8 * x] >= 128 ? 1 : 0;
   }
 }
 
@@ -862,9 +940,10 @@ extern "C" int ih_euler_cfg_step(const void* noise_pred, void* latents, void* mo
   cudaStream_t stream = (cudaStream_t)stream_;
   IH_CHECK(noise_pred && latents && model_in && sigmas && step, IH_ERR_ARG, "ih_euler_cfg_step: null pointer");
   const long long total = n_per_image * n_images;
-  IH_CUDA(launch_kernel(euler_cfg_kernel, dim3(grid_for(total, 256)), dim3(256), (size_t)(0), stream, (const __half*)noise_pred, (__half*)latents,
+  IH_CUDA(launch_kernel(euler_cfg_kernel<false>, dim3(grid_for(total, 256)), dim3(256), (size_t)(0), stream, (const __half*)noise_pred, (__half*)latents,
                                                              (__half*)model_in, (const float*)sigmas,
-                                                             (const int*)step, guidance, n_per_image, n_images));
+                                                             (const int*)step, guidance, n_per_image, n_images,
+                                                             InpaintBlend{}));
   IH_CUDA(launch_kernel(step_inc_kernel, dim3(1), dim3(1), (size_t)(0), stream, (int*)step));
   return 0;
 }
@@ -876,9 +955,36 @@ extern "C" int ih_euler_step_ex(const void* noise_pred, void* latents, void* mod
   IH_CHECK(noise_pred && latents && model_in && sigmas && step, IH_ERR_ARG, "ih_euler_step_ex: null pointer");
   IH_CHECK(n_per_image > 1 && n_images > 0, IH_ERR_SHAPE, "ih_euler_step_ex: bad shape");
   IH_CHECK(guidance_rescale >= 0.f && guidance_rescale <= 1.f, IH_ERR_ARG, "ih_euler_step_ex: guidance_rescale outside [0, 1]");
-  IH_CUDA(launch_kernel(euler_ex_kernel, dim3(n_images), dim3(1024), (size_t)(0), stream, (const __half*)noise_pred,
+  IH_CUDA(launch_kernel(euler_ex_kernel<false>, dim3(n_images), dim3(1024), (size_t)(0), stream, (const __half*)noise_pred,
                         (__half*)latents, (__half*)model_in, (const float*)sigmas, (const int*)step, guidance,
-                        guidance_rescale, n_per_image, n_images, use_cfg ? 1 : 0));
+                        guidance_rescale, n_per_image, n_images, use_cfg ? 1 : 0, InpaintBlend{}));
+  IH_CUDA(launch_kernel(step_inc_kernel, dim3(1), dim3(1), (size_t)(0), stream, (int*)step));
+  return 0;
+}
+
+extern "C" int ih_euler_step_inpaint(const void* noise_pred, void* latents, void* model_in, const void* sigmas,
+                                     void* step, float guidance, float guidance_rescale, long long n_per_image,
+                                     int n_images, int use_cfg, const void* mask_u8, int Bm, long long hw,
+                                     const void* z0, const void* noise, const void* last_step, void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  IH_CHECK(noise_pred && latents && model_in && sigmas && step && mask_u8 && z0 && noise && last_step, IH_ERR_ARG,
+           "ih_euler_step_inpaint: null pointer");
+  IH_CHECK(n_per_image > 1 && n_images > 0 && hw > 0 && n_per_image % hw == 0 && Bm > 0 && n_images % Bm == 0,
+           IH_ERR_SHAPE, "ih_euler_step_inpaint: bad shape (n_per_image %% hw == 0 and n_images %% Bm == 0 are required)");
+  IH_CHECK(guidance_rescale >= 0.f && guidance_rescale <= 1.f, IH_ERR_ARG,
+           "ih_euler_step_inpaint: guidance_rescale outside [0, 1]");
+  const InpaintBlend bl{(const unsigned char*)mask_u8, (const __half*)z0, (const __half*)noise, (const int*)last_step,
+                        hw, Bm};
+  if (use_cfg && guidance_rescale == 0.f) {
+    const long long total = n_per_image * n_images;
+    IH_CUDA(launch_kernel(euler_cfg_kernel<true>, dim3(grid_for(total, 256)), dim3(256), (size_t)(0), stream,
+                          (const __half*)noise_pred, (__half*)latents, (__half*)model_in, (const float*)sigmas,
+                          (const int*)step, guidance, n_per_image, n_images, bl));
+  } else {
+    IH_CUDA(launch_kernel(euler_ex_kernel<true>, dim3(n_images), dim3(1024), (size_t)(0), stream,
+                          (const __half*)noise_pred, (__half*)latents, (__half*)model_in, (const float*)sigmas,
+                          (const int*)step, guidance, guidance_rescale, n_per_image, n_images, use_cfg ? 1 : 0, bl));
+  }
   IH_CUDA(launch_kernel(step_inc_kernel, dim3(1), dim3(1), (size_t)(0), stream, (int*)step));
   return 0;
 }
@@ -1031,8 +1137,34 @@ extern "C" int ih_vae_sample_add_noise_f16(const void* moments, long long ldm, i
   IH_CHECK(!eps_f32 || (Be > 0 && B % Be == 0), IH_ERR_SHAPE, "ih_vae_sample_add_noise_f16: B %% Be != 0");
   const long long HW = (long long)h * w;
   const long long total = (long long)B * C * HW;
-  IH_CUDA(launch_kernel(vae_sample_add_noise_kernel, dim3(grid_for(total, 256)), dim3(256), (size_t)0, (cudaStream_t)stream,
-                        (const __half*)moments, ldm, Bm, (const float*)eps_f32, Be, (const __half*)noise,
-                        (__half*)out_nchw, B, C, HW, scaling_factor, sigma));
+  IH_CUDA(launch_kernel(vae_sample_add_noise_kernel<false>, dim3(grid_for(total, 256)), dim3(256), (size_t)0,
+                        (cudaStream_t)stream, (const __half*)moments, ldm, Bm, (const float*)eps_f32, Be,
+                        (const __half*)noise, (__half*)out_nchw, B, C, HW, scaling_factor, sigma, (__half*)nullptr, 0));
+  return 0;
+}
+
+extern "C" int ih_vae_sample_inpaint_f16(const void* moments, long long ldm, int Bm, const void* eps_f32, int Be,
+                                         const void* noise, void* latents_nchw, void* z0_nchw, int B, int C, int h,
+                                         int w, float scaling_factor, float sigma, int pure_noise, void* stream) {
+  IH_CHECK(moments && noise && latents_nchw && z0_nchw, IH_ERR_ARG, "ih_vae_sample_inpaint_f16: null pointer");
+  IH_CHECK(B > 0 && C > 0 && h > 0 && w > 0 && Bm > 0 && B % Bm == 0 && ldm >= (eps_f32 ? 2 * C : C), IH_ERR_SHAPE,
+           "ih_vae_sample_inpaint_f16: bad shape (B %% Bm == 0 and ldm >= 2C with eps, >= C without are required)");
+  IH_CHECK(!eps_f32 || (Be > 0 && B % Be == 0), IH_ERR_SHAPE, "ih_vae_sample_inpaint_f16: B %% Be != 0");
+  const long long HW = (long long)h * w;
+  const long long total = (long long)B * C * HW;
+  IH_CUDA(launch_kernel(vae_sample_add_noise_kernel<true>, dim3(grid_for(total, 256)), dim3(256), (size_t)0,
+                        (cudaStream_t)stream, (const __half*)moments, ldm, Bm, (const float*)eps_f32, Be,
+                        (const __half*)noise, (__half*)latents_nchw, B, C, HW, scaling_factor, sigma, (__half*)z0_nchw,
+                        pure_noise ? 1 : 0));
+  return 0;
+}
+
+extern "C" int ih_latent_mask_u8(const void* mask_u8, void* out_u8, int Bm, int H, int W, void* stream) {
+  IH_CHECK(mask_u8 && out_u8, IH_ERR_ARG, "ih_latent_mask_u8: null pointer");
+  IH_CHECK(Bm > 0 && H > 0 && W > 0 && H % 8 == 0 && W % 8 == 0, IH_ERR_SHAPE,
+           "ih_latent_mask_u8: bad shape (H and W must be positive multiples of 8)");
+  const long long total = (long long)Bm * (H / 8) * (W / 8);
+  IH_CUDA(launch_kernel(latent_mask_u8_kernel, dim3(grid_for(total, 256)), dim3(256), (size_t)0, (cudaStream_t)stream,
+                        (const unsigned char*)mask_u8, (unsigned char*)out_u8, Bm, H, W));
   return 0;
 }

@@ -9,12 +9,15 @@ Loop options of the reference that are honoured here (all graph-replayed; a call
 not the graph): classifier-free guidance on or off (`guidance_scale <= 1`, :223,:332,:348), `guidance_rescale`
 (:352-354), `denoising_end` (:307-316, via `num_loop_steps`), `callback` / `callback_steps` (:359-363),
 `control_guidance_start/end` IP-scale gating (:326-329), negative micro-conditioning time ids (:286-300).
+Inpainting (`inpaint=`) blends the latents with the source image's inside the same Euler kernel, so a masked step
+launches as many kernels as a plain one.
 
 Graph lifetime: a captured graph holds raw pointers.  Everything it reads lives in buffers that are owned per shape
-and never freed while the graph exists -- the engine's static inputs (`_static`), the processors' K/V buffers and the
-UNet's add-embedding buffer (per-shape dicts inside those objects), and the library's grow-only scratch buffers whose
-re-allocation bumps `ops.workspace_generation()`.  A graph is replayed only if it was captured under the current UNet
-`graph_epoch` (weights / processors unchanged) and the current workspace generation; otherwise it is re-captured.
+and never freed while the graph exists -- the engine's static inputs (`_static`, and `_inpaint_static` for the
+mask, z0, noise and last-step index), the processors' K/V buffers and the UNet's add-embedding buffer (per-shape
+dicts inside those objects), and the library's grow-only scratch buffers whose re-allocation bumps
+`ops.workspace_generation()`.  A graph is replayed only if it was captured under the current UNet `graph_epoch`
+(weights / processors unchanged) and the current workspace generation; otherwise it is re-captured.
 """
 from __future__ import annotations
 
@@ -37,6 +40,7 @@ class DenoiseEngine:
         self.use_cuda_graph = use_cuda_graph and self.device.type == "cuda"
         self._graphs: Dict[Tuple, Tuple[torch.cuda.CUDAGraph, int]] = {}   # key -> (graph, workspace generation)
         self._static: Dict[Tuple, dict] = {}
+        self._inpaint_static: Dict[Tuple, dict] = {}
         self._tables: Dict[int, Tuple[torch.Tensor, torch.Tensor, float]] = {}
         self._epoch = getattr(unet, "graph_epoch", 0)
         self.last_launches_per_step = 0
@@ -79,10 +83,29 @@ class DenoiseEngine:
             self._static[key] = st
         return st
 
-    def _step(self, st, timesteps, sigmas, guidance, use_cfg=True, rescale=0.0):
+    def _inpaint_buffers(self, n: int, h: int, w: int, n_masks: int):
+        key = (n, h, w, n_masks)
+        bs = self._inpaint_static.get(key)
+        if bs is None:
+            dev = self.device
+            L = self.unet.config.in_channels
+            bs = {
+                "mask": torch.empty((n_masks, h, w), dtype=torch.uint8, device=dev),
+                "z0": torch.empty((n, L, h, w), dtype=torch.float16, device=dev),
+                "noise": torch.empty((n, L, h, w), dtype=torch.float16, device=dev),
+                "last": torch.zeros((1,), dtype=torch.int32, device=dev),
+            }
+            self._inpaint_static[key] = bs
+        return bs
+
+    def _step(self, st, timesteps, sigmas, guidance, use_cfg=True, rescale=0.0, blend=None):
         noise = self.unet(st["model_in"], timesteps, st["ehs"], st["text_embeds"], st["time_ids"], step=st["step"])
-        ops.euler_step(noise, st["latents"], st["model_in"], sigmas, st["step"], guidance, use_cfg=use_cfg,
-                       guidance_rescale=rescale)
+        if blend is None:
+            ops.euler_step(noise, st["latents"], st["model_in"], sigmas, st["step"], guidance, use_cfg=use_cfg,
+                           guidance_rescale=rescale)
+        else:
+            ops.euler_step_inpaint(noise, st["latents"], st["model_in"], sigmas, st["step"], guidance, blend["mask"],
+                                   blend["z0"], blend["noise"], blend["last"], use_cfg=use_cfg, guidance_rescale=rescale)
 
     # ------------------------------------------------------------------------------------------------------------
     @torch.no_grad()
@@ -92,7 +115,8 @@ class DenoiseEngine:
             control_guidance_start: float = 0.0, control_guidance_end: float = 1.0, stop_after: Optional[int] = None,
             start_step: int = 0, guidance_rescale: float = 0.0, num_loop_steps: Optional[int] = None,
             callback: Optional[Callable] = None, callback_steps: int = 1,
-            negative_time_ids: Optional[torch.Tensor] = None, count_from_start: bool = False) -> torch.Tensor:
+            negative_time_ids: Optional[torch.Tensor] = None, count_from_start: bool = False,
+            inpaint: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None) -> torch.Tensor:
         """latents [n,4,h,w] (already scaled by init_noise_sigma; host or device); embeds host or device tensors.
         Returns the latents after the last executed step as a new device tensor.
 
@@ -105,7 +129,13 @@ class DenoiseEngine:
         `count_from_start=True` is img2img (`start_step` = t_start of `strength`, the latents noised to sigma[t_start]):
         the control_guidance_start/end fractions and the callback's step index then count the executed steps from 0 over
         the truncated list (steps start_step .. loop end), as `enumerate(timesteps)` does in [3P] diffusers' img2img
-        loop.  The default counts from the start of the full schedule (a resumed PNS trajectory)."""
+        loop.  The default counts from the start of the full schedule (a resumed PNS trajectory).
+
+        `inpaint=(mask, z0, noise)` is masked inpainting ([3P] diffusers StableDiffusionXLInpaintPipeline, 4-channel
+        UNet): mask uint8 {0, 1} [Bm, h, w] (1 = regenerate; latent image b uses mask b % Bm), z0 and noise fp16
+        [n, 4, h, w].  After every step the latents outside the mask become z0 noised to the next sigma, and z0 itself
+        after the last step of the loop (num_loop_steps - 1); the next model_in and the callback see the blended
+        latents."""
         use_cfg = guidance_scale > 1.0                                            # :223
         if use_cfg and (negative_prompt_embeds is None or negative_pooled is None):
             raise IHError("classifier-free guidance needs negative_prompt_embeds / negative_pooled")
@@ -135,6 +165,18 @@ class DenoiseEngine:
         if not 0 <= start_step <= loop_T:
             raise IHError(f"start_step {start_step} outside the {loop_T}-step loop")
         st["step"].fill_(start_step)
+        blend = None
+        if inpaint is not None:
+            mask, z0, noise = inpaint
+            if mask.dim() != 3 or tuple(mask.shape[1:]) != (h, w) or n % mask.shape[0] \
+                    or tuple(z0.shape) != tuple(latents.shape) or tuple(noise.shape) != tuple(latents.shape):
+                raise IHError(f"inpaint: mask [Bm, {h}, {w}] with {n} % Bm == 0, z0 and noise {tuple(latents.shape)} "
+                              "required")
+            blend = self._inpaint_buffers(n, h, w, mask.shape[0])
+            blend["mask"].copy_(mask, non_blocking=True)
+            blend["z0"].copy_(z0, non_blocking=True)
+            blend["noise"].copy_(noise, non_blocking=True)
+            blend["last"].fill_(loop_T - 1)
         self.unet.prepare_conditioning(st["ehs"], st["text_embeds"], st["time_ids"])
         ops.scale_model_input(st["latents"], st["model_in"], sigmas, st["step"], duplicate=use_cfg)   # :332-334
 
@@ -148,7 +190,8 @@ class DenoiseEngine:
             return 0.0 if off else float(ip_scale)
 
         def gkey(scale: float):
-            return (n, h, w, L, T, use_cfg, float(guidance_scale), rescale, scale)
+            key = (n, h, w, L, T, use_cfg, float(guidance_scale), rescale, scale)
+            return key if blend is None else key + ("inpaint", blend["mask"].shape[0])
 
         if self.use_cuda_graph:
             if self._epoch != getattr(self.unet, "graph_epoch", 0):       # weights / processors changed since capture
@@ -163,7 +206,7 @@ class DenoiseEngine:
                     break
                 for sc in missing:
                     self.set_scale(sc)
-                    g = self._capture(st, timesteps, sigmas, guidance_scale, use_cfg, rescale)
+                    g = self._capture(st, timesteps, sigmas, guidance_scale, use_cfg, rescale, blend)
                     self._graphs[gkey(sc)] = (g, ops.workspace_generation())
                     captured = True
             else:
@@ -179,27 +222,27 @@ class DenoiseEngine:
                 self._graphs[gkey(sc)][0].replay()
             else:
                 self.set_scale(sc)
-                self._step(st, timesteps, sigmas, guidance_scale, use_cfg, rescale)
+                self._step(st, timesteps, sigmas, guidance_scale, use_cfg, rescale, blend)
             if callback is not None and (i - origin) % callback_steps == 0:       # :359-363 (Euler: order 1, no warm-up)
                 callback(i - origin, timesteps[i], st["latents"])
         self.set_scale(ip_scale)
         return st["latents"].clone()
 
-    def _capture(self, st, timesteps, sigmas, guidance, use_cfg=True, rescale=0.0):
+    def _capture(self, st, timesteps, sigmas, guidance, use_cfg=True, rescale=0.0, blend=None):
         # warm-up on a side stream (sets kernel attributes, fills the TMA descriptor cache, sizes the allocator and
         # the library's scratch buffers)
         side = torch.cuda.Stream(device=self.device)
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):
             st["step"].zero_()
-            self._step(st, timesteps, sigmas, guidance, use_cfg, rescale)
+            self._step(st, timesteps, sigmas, guidance, use_cfg, rescale, blend)
         torch.cuda.current_stream().wait_stream(side)
         torch.cuda.synchronize()
         st["step"].zero_()
         g = torch.cuda.CUDAGraph()
         before = ops.launch_count()
         with torch.cuda.graph(g):
-            self._step(st, timesteps, sigmas, guidance, use_cfg, rescale)
+            self._step(st, timesteps, sigmas, guidance, use_cfg, rescale, blend)
         self.last_launches_per_step = ops.launch_count() - before
         self.graphs_captured += 1
         return g

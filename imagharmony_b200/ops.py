@@ -6,7 +6,7 @@ PyTorch/CPU fallback: a CPU tensor or a missing library raises.
 from __future__ import annotations
 
 import os
-from typing import Optional
+from typing import Optional, Tuple
 
 import torch
 
@@ -229,6 +229,43 @@ def vae_sample_add_noise(moments: torch.Tensor, eps: Optional[torch.Tensor], noi
     check(lib.ih_vae_sample_add_noise_f16(moments.data_ptr(), ldm, Bm, _p(eps), Be, noise.data_ptr(), out.data_ptr(), B,
                                           channels, h, w, float(scaling_factor), float(sigma), _stream()),
           "ih_vae_sample_add_noise_f16")
+    return out
+
+
+def vae_sample_inpaint(moments: torch.Tensor, eps: Optional[torch.Tensor], noise: torch.Tensor, channels: int,
+                       scaling_factor: float, sigma: float, pure_noise: bool) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Inpainting start latents and z0 (both NCHW fp16 [B, C, h, w]), arguments as vae_sample_add_noise:
+    z0 = fp16(sf * fp16(mean + std * eps)); latents = fp16(z0 + fp16(noise * fp16(sigma))), or with `pure_noise`
+    (strength 1) fp16(noise * sigma) with sigma = init_noise_sigma."""
+    lib = _lib.load()
+    _req(moments, "moments"); _req(noise, "noise")
+    Bm, h, w, ldm = moments.shape
+    B = noise.shape[0]
+    if not moments.is_contiguous() or not noise.is_contiguous() or tuple(noise.shape) != (B, channels, h, w):
+        raise IHError(f"vae_sample_inpaint: contiguous moments and noise [B, {channels}, {h}, {w}] required")
+    Be = 0
+    if eps is not None:
+        _req(eps, "eps", torch.float32)
+        Be = eps.shape[0]
+        if not eps.is_contiguous() or tuple(eps.shape[1:]) != (channels, h, w):
+            raise IHError(f"vae_sample_inpaint: eps must be contiguous [Be, {channels}, {h}, {w}]")
+    latents = torch.empty((B, channels, h, w), dtype=torch.float16, device=moments.device)
+    z0 = torch.empty_like(latents)
+    check(lib.ih_vae_sample_inpaint_f16(moments.data_ptr(), ldm, Bm, _p(eps), Be, noise.data_ptr(), latents.data_ptr(),
+                                        z0.data_ptr(), B, channels, h, w, float(scaling_factor), float(sigma),
+                                        int(pure_noise), _stream()), "ih_vae_sample_inpaint_f16")
+    return latents, z0
+
+
+def latent_mask(mask_u8: torch.Tensor) -> torch.Tensor:
+    """uint8 grayscale mask [Bm, H, W] (H, W multiples of 8) -> uint8 {0, 1} [Bm, H/8, W/8]: pixel (8y, 8x) >= 128."""
+    lib = _lib.load()
+    _req(mask_u8, "mask_u8", torch.uint8)
+    if mask_u8.dim() != 3 or not mask_u8.is_contiguous():
+        raise IHError("latent_mask: contiguous uint8 [Bm, H, W] required")
+    Bm, H, W = mask_u8.shape
+    out = torch.empty((Bm, H // 8, W // 8), dtype=torch.uint8, device=mask_u8.device)
+    check(lib.ih_latent_mask_u8(mask_u8.data_ptr(), out.data_ptr(), Bm, H, W, _stream()), "ih_latent_mask_u8")
     return out
 
 
@@ -621,6 +658,31 @@ def euler_step(noise_pred: torch.Tensor, latents: torch.Tensor, model_in: torch.
     check(lib.ih_euler_step_ex(noise_pred.data_ptr(), latents.data_ptr(), model_in.data_ptr(), sigmas.data_ptr(),
                                step.data_ptr(), float(guidance), float(guidance_rescale), per, n, int(use_cfg),
                                _stream()), "ih_euler_step_ex")
+
+
+def euler_step_inpaint(noise_pred: torch.Tensor, latents: torch.Tensor, model_in: torch.Tensor, sigmas: torch.Tensor,
+                       step: torch.Tensor, guidance: float, mask: torch.Tensor, z0: torch.Tensor, noise: torch.Tensor,
+                       last: torch.Tensor, *, use_cfg: bool = True, guidance_rescale: float = 0.0) -> None:
+    """euler_step followed by the inpainting blend, in the same kernel (`ih_euler_step_inpaint`): outside the mask the
+    latents become z0 noised to the next sigma (z0 itself on the step index `last`), before model_in is formed.
+    mask uint8 {0, 1} [Bm, h, w] (latent image b uses mask b % Bm); z0, noise fp16 like `latents`; last int32 [1]."""
+    lib = _lib.load()
+    _req(noise_pred, "noise_pred"); _req(latents, "latents"); _req(model_in, "model_in")
+    _req(sigmas, "sigmas", torch.float32); _req(step, "step", torch.int32)
+    _req(mask, "mask", torch.uint8); _req(z0, "z0"); _req(noise, "noise"); _req(last, "last", torch.int32)
+    n, _, h, w = latents.shape
+    per = latents.numel() // n
+    want = (2 * n if use_cfg else n) * per
+    if noise_pred.numel() != want or model_in.numel() != want:
+        raise IHError(f"euler_step_inpaint: noise_pred / model_in must hold {want} elements (use_cfg={use_cfg})")
+    if z0.shape != latents.shape or noise.shape != latents.shape or mask.dim() != 3 or tuple(mask.shape[1:]) != (h, w) \
+            or n % mask.shape[0] or not (mask.is_contiguous() and z0.is_contiguous() and noise.is_contiguous()):
+        raise IHError(f"euler_step_inpaint: contiguous z0 / noise {tuple(latents.shape)} and mask [Bm, {h}, {w}] with "
+                      f"{n} % Bm == 0 required")
+    check(lib.ih_euler_step_inpaint(noise_pred.data_ptr(), latents.data_ptr(), model_in.data_ptr(), sigmas.data_ptr(),
+                                    step.data_ptr(), float(guidance), float(guidance_rescale), per, n, int(use_cfg),
+                                    mask.data_ptr(), mask.shape[0], h * w, z0.data_ptr(), noise.data_ptr(),
+                                    last.data_ptr(), _stream()), "ih_euler_step_inpaint")
 
 
 def scale_model_input(latents: torch.Tensor, model_in: torch.Tensor, sigmas: torch.Tensor, step: torch.Tensor,

@@ -207,6 +207,15 @@ int ih_image_im2col3x3_u8(const void* rgb_u8, void* out, int B, int H, int W, in
 int ih_vae_sample_add_noise_f16(const void* moments, long long ldm, int Bm, const void* eps_f32, int Be, const void* noise,
                                 void* out_nchw, int B, int C, int h, int w, float scaling_factor, float sigma,
                                 void* stream);
+/* Inpainting start latents: as ih_vae_sample_add_noise_f16, and z0_nchw receives z (fp16 NCHW [B, C, h, w], the
+ * blend's clean latents).  pure_noise = 1 (strength 1): latents = fp16(noise * sigma), sigma = init_noise_sigma, not
+ * rounded to fp16. */
+int ih_vae_sample_inpaint_f16(const void* moments, long long ldm, int Bm, const void* eps_f32, int Be, const void* noise,
+                              void* latents_nchw, void* z0_nchw, int B, int C, int h, int w, float scaling_factor,
+                              float sigma, int pure_noise, void* stream);
+/* Inpainting latent mask: uint8 grayscale [Bm, H, W] (H, W multiples of 8) -> uint8 {0, 1} [Bm, H/8, W/8], latent
+ * (y, x) = pixel (8y, 8x) >= 128 ([3P] VaeImageProcessor binarize at 0.5, then F.interpolate nearest). */
+int ih_latent_mask_u8(const void* mask_u8, void* out_u8, int Bm, int H, int W, void* stream);
 /* conv_out on ih_conv2d_f16 with Cout padded to 16: gather NHWC [B, HW, ldc] channels [0, C) into NCHW [B, C, HW]. */
 int ih_nhwc_to_nchw_f16(const void* x, long long ldc, void* out, int B, long long HW, int C, void* stream);
 
@@ -248,6 +257,18 @@ int ih_resize_patchify_f16(const void* img_nchw, void* out, int B, int C, int Hi
 int ih_euler_step_ex(const void* noise_pred, void* latents, void* model_in, const void* sigmas, void* step,
                      float guidance, float guidance_rescale, long long n_per_image, int n_images, int use_cfg,
                      void* stream);
+
+/* Masked (inpainting) scheduler transition ([3P] diffusers StableDiffusionXLInpaintPipeline, 4-channel UNet): the
+ * transition of ih_euler_cfg_step (use_cfg && guidance_rescale == 0) or ih_euler_step_ex (otherwise), then, with k the
+ * step index read from `step`, before model_in is formed:
+ *   proper  = z0 if k == *last_step, else fp16(z0 + fp16(noise * fp16(sigma_{k+1})))   (add_noise at the next sigma);
+ *   latents = fp16(fp16(fp16(1 - m) * proper) + fp16(m * latents)).
+ * mask_u8: uint8 {0, 1} [Bm, hw] (1 = regenerate), latent image b uses mask b % Bm; z0, noise: fp16 NCHW, the latents'
+ * shape; last_step: device int32, the index of the last executed step.  Launches as many kernels as the plain step. */
+int ih_euler_step_inpaint(const void* noise_pred, void* latents, void* model_in, const void* sigmas, void* step,
+                          float guidance, float guidance_rescale, long long n_per_image, int n_images, int use_cfg,
+                          const void* mask_u8, int Bm, long long hw, const void* z0, const void* noise,
+                          const void* last_step, void* stream);
 
 /* model_in = cat([latents, latents]) / sqrt(sigma[*step]^2 + 1)   (custom_pipelines.py:332-334, first step). */
 int ih_scale_model_input(const void* latents, void* model_in, const void* sigmas, const void* step, long long total,

@@ -418,14 +418,7 @@ class StableDiffusionXLImg2ImgCustomPipeline(StableDiffusionXLCustomPipeline):
         requires_aesthetics_score = false, so its time ids equal the text-to-image ones)."""
         if image is None:
             raise ValueError("img2img needs a source `image`")
-        if not 0.0 <= strength <= 1.0:
-            raise ValueError(f"The value of strength should be in [0.0, 1.0] but is {strength}")
-        if callback is not None and (not isinstance(callback_steps, int) or callback_steps <= 0):
-            raise ValueError(f"`callback_steps` has to be a positive integer but is {callback_steps}")
-        t_start, n_exec = self.get_timesteps(num_inference_steps, strength)
-        if n_exec < 1:
-            raise ValueError(f"strength {strength} with num_inference_steps {num_inference_steps} leaves no denoising "
-                             "step (the number of steps run is min(int(num_inference_steps * strength), num_inference_steps))")
+        t_start = self._check_edit_args(strength, num_inference_steps, callback, callback_steps)
         do_classifier_free_guidance = guidance_scale > 1.0
         (prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds, negative_pooled_prompt_embeds) = \
             self.encode_prompt(prompt, prompt_2, None, num_images_per_prompt, do_classifier_free_guidance,
@@ -435,8 +428,37 @@ class StableDiffusionXLImg2ImgCustomPipeline(StableDiffusionXLCustomPipeline):
         self.scheduler.set_timesteps(num_inference_steps)
         sigma = float(self.scheduler.sigmas[t_start])                   # add_noise at the begin index t_start
         lat, size = self.prepare_img2img_latents(image, batch, generator, sigma)
-        original_size = original_size or size
-        target_size = target_size or size
+        return self._denoise_and_decode(
+            lat, t_start, num_inference_steps, (prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds,
+                                                negative_pooled_prompt_embeds),
+            guidance_scale=guidance_scale, denoising_end=denoising_end, guidance_rescale=guidance_rescale,
+            original_size=original_size or size, crops_coords_top_left=crops_coords_top_left,
+            target_size=target_size or size, negative_original_size=negative_original_size,
+            negative_crops_coords_top_left=negative_crops_coords_top_left, negative_target_size=negative_target_size,
+            control_guidance_start=control_guidance_start, control_guidance_end=control_guidance_end,
+            callback=callback, callback_steps=callback_steps, output_type=output_type, return_dict=return_dict)
+
+    def _check_edit_args(self, strength: float, num_inference_steps: int, callback, callback_steps) -> int:
+        """Validates the editing arguments; -> t_start."""
+        if not 0.0 <= strength <= 1.0:
+            raise ValueError(f"The value of strength should be in [0.0, 1.0] but is {strength}")
+        if callback is not None and (not isinstance(callback_steps, int) or callback_steps <= 0):
+            raise ValueError(f"`callback_steps` has to be a positive integer but is {callback_steps}")
+        t_start, n_exec = self.get_timesteps(num_inference_steps, strength)
+        if n_exec < 1:
+            raise ValueError(f"strength {strength} with num_inference_steps {num_inference_steps} leaves no denoising "
+                             "step (the number of steps run is min(int(num_inference_steps * strength), num_inference_steps))")
+        return t_start
+
+    def _denoise_and_decode(self, lat, t_start: int, num_inference_steps: int, embeds, *, guidance_scale,
+                            denoising_end, guidance_rescale, original_size, crops_coords_top_left, target_size,
+                            negative_original_size, negative_crops_coords_top_left, negative_target_size,
+                            control_guidance_start, control_guidance_end, callback, callback_steps, output_type,
+                            return_dict, inpaint=None):
+        """The editing loop from t_start (gating and callback counted over the executed steps) and the decode tail;
+        `inpaint` is DenoiseEngine.run's."""
+        prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds, negative_pooled_prompt_embeds = embeds
+        batch = prompt_embeds.shape[0]
 
         def time_ids(size, crop, target):
             return torch.tensor([list(size) + list(crop) + list(target)], dtype=torch.float32).repeat(batch, 1)
@@ -462,7 +484,7 @@ class StableDiffusionXLImg2ImgCustomPipeline(StableDiffusionXLCustomPipeline):
                                   control_guidance_end=control_guidance_end, guidance_rescale=guidance_rescale,
                                   start_step=t_start, num_loop_steps=loop_steps, callback=callback,
                                   callback_steps=callback_steps, negative_time_ids=negative_add_time_ids,
-                                  count_from_start=True)
+                                  count_from_start=True, inpaint=inpaint)
         else:
             out = lat
         self.set_scale(conditioning_scale)
@@ -479,3 +501,134 @@ class StableDiffusionXLImg2ImgCustomPipeline(StableDiffusionXLCustomPipeline):
         if not return_dict:
             return (image,)
         return StableDiffusionXLPipelineOutput(images=image)
+
+
+class StableDiffusionXLInpaintCustomPipeline(StableDiffusionXLImg2ImgCustomPipeline):
+    """Masked inpainting on the img2img call surface: `image=` (the source), `mask_image=` (white = regenerate) and
+    `strength=`, following [3P] diffusers==0.30.0 `StableDiffusionXLInpaintPipeline` with the 4-channel SDXL-base UNet
+    (the rules are stated in oracle/inpaint_ref.py).  Unlike img2img, the output size is `height` x `width` (default
+    unet sample_size * 8) and the source image is resized to it.  After every denoising step the latents outside the
+    mask are replaced by the source image's latents noised to the next sigma; the replacement runs inside the Euler
+    kernel of the CUDA-graph loop (`DenoiseEngine.run(inpaint=...)`).  IPAdapterXL.generate(image=..., mask_image=...)
+    reaches this call through its **kwargs; `pil_image` stays the IP reference."""
+
+    def preprocess_mask(self, mask_image, height: int, width: int) -> torch.Tensor:
+        """-> uint8 grayscale mask [Bm, height, width] on the device.  PIL masks are converted to "L" and
+        Lanczos-resized to (width, height); a float tensor [H, W], [B, H, W] or [B, 1, H, W] with values in [0, 1] must
+        already be (height, width) and is binarized at 0.5 here (to 255 / 0)."""
+        import numpy as np
+        from PIL import Image
+        if isinstance(mask_image, torch.Tensor):
+            m = mask_image.float()
+            m = m[None] if m.dim() == 2 else (m[:, 0] if m.dim() == 4 and m.shape[1] == 1 else m)
+            if m.dim() != 3 or tuple(m.shape[1:]) != (height, width):
+                raise ValueError(f"a tensor mask must be [H, W], [B, H, W] or [B, 1, H, W] with (H, W) = "
+                                 f"({height}, {width}), got {tuple(mask_image.shape)}")
+            if m.numel() and (m.min() < 0 or m.max() > 1):
+                raise ValueError("a tensor mask must have values in [0, 1]")
+            return torch.where(m >= 0.5, 255, 0).to(device=self.device, dtype=torch.uint8).contiguous()
+        if isinstance(mask_image, Image.Image) or (isinstance(mask_image, (list, tuple)) and mask_image
+                                                   and all(isinstance(m, Image.Image) for m in mask_image)):
+            arrs = []
+            for im in [mask_image] if isinstance(mask_image, Image.Image) else list(mask_image):
+                im = im.convert("L")
+                if im.size != (width, height):
+                    im = im.resize((width, height), resample=Image.LANCZOS)
+                arrs.append(np.asarray(im, dtype=np.uint8))
+            return torch.from_numpy(np.stack(arrs)).to(self.device)
+        raise TypeError(f"mask_image must be a PIL image, a list of PIL images or a torch tensor, got {type(mask_image)}")
+
+    def prepare_inpaint_latents(self, image, mask_image, batch: int, generator, height: int, width: int, t_start: int,
+                                is_strength_max: bool):
+        """-> (start latents [batch, 4, h, w] fp16, (latent mask uint8 {0, 1} [Bm, h, w], z0, noise)), the second item
+        being DenoiseEngine.run's `inpaint`.  Call after scheduler.set_timesteps.
+
+        Draw order ([3P] prepare_latents with a 4-channel UNet): the posterior eps (fp32) and then the noise (fp16).  With
+        a generator list, source image i draws its eps from generator[i] for i < n_img only -- the images are encoded as
+        they are, not replicated to the batch as in img2img -- and batch slot b then draws its noise from generator[b]."""
+        from PIL import Image
+        if isinstance(image, (Image.Image, list, tuple)):
+            images = [image] if isinstance(image, Image.Image) else list(image)
+            if not all(isinstance(im, Image.Image) for im in images):
+                raise TypeError("image must be a PIL image, a list of PIL images or a torch tensor")
+            image = [im if im.size == (width, height) else im.convert("RGB").resize((width, height), resample=Image.LANCZOS)
+                     for im in images]                          # preprocess_image converts the rest to RGB
+        kind, x = self.preprocess_image(image)
+        h, w = height // self.vae_scale_factor, width // self.vae_scale_factor
+        have = tuple(x.shape[2:]) if kind != "pixels" else tuple(x.shape[1:3])
+        if have != ((h, w) if kind == "latents" else (height, width)):
+            raise ValueError(f"a tensor image must match height x width = {height} x {width}, got {tuple(x.shape)}")
+        n_img = x.shape[0]
+        if batch % n_img:
+            raise ValueError(f"cannot duplicate {n_img} source images to a batch of {batch}")
+        if isinstance(generator, list) and len(generator) != batch:
+            raise ValueError(f"got {len(generator)} generators for a batch of {batch}")
+        mask_u8 = self.preprocess_mask(mask_image, height, width)
+        if batch % mask_u8.shape[0]:
+            raise ValueError(f"{mask_u8.shape[0]} masks do not divide the batch of {batch}")
+        L = self.unet.config.in_channels
+
+        def randn(shape, g, dtype):
+            return torch.randn(shape, generator=g, device=g.device if g is not None else "cpu", dtype=dtype)
+        if kind == "latents":
+            moments, eps = x.permute(0, 2, 3, 1).contiguous(), None
+        else:
+            if self.vae_encoder is None:
+                raise IHError("this pipeline has no VAE encoder: build it with from_random(vae_cfg=...) or from_pretrained "
+                              "with a vae/ folder, or pass latents as a 4-channel image tensor")
+            moments = self.vae_encoder.encode(x)
+            if isinstance(generator, list):
+                eps = torch.cat([randn((1, L, h, w), generator[i], torch.float32).to(self.device) for i in range(n_img)])
+            else:
+                eps = randn((n_img, L, h, w), generator, torch.float32).to(self.device)
+        if isinstance(generator, list):
+            noise = torch.cat([randn((1, L, h, w), g, torch.float16).to(self.device) for g in generator], dim=0)
+        else:
+            noise = randn((batch, L, h, w), generator, torch.float16).to(self.device)
+        from imagharmony_b200 import ops
+        sf = 1.0 if eps is None else self.vae_encoder.config.scaling_factor
+        sigma = float(self.scheduler.init_noise_sigma if is_strength_max else self.scheduler.sigmas[t_start])
+        lat, z0 = ops.vae_sample_inpaint(moments, eps, noise, L, sf, sigma, is_strength_max)
+        return lat, (ops.latent_mask(mask_u8), z0, noise)
+
+    @torch.no_grad()
+    def __call__(self, prompt: Optional[Union[str, List[str]]] = None, prompt_2=None, image=None, mask_image=None,
+                 height: Optional[int] = None, width: Optional[int] = None, strength: float = 0.9999,
+                 num_inference_steps: int = 50, denoising_end: Optional[float] = None, guidance_scale: float = 5.0,
+                 negative_prompt=None, negative_prompt_2=None, num_images_per_prompt: Optional[int] = 1,
+                 eta: float = 0.0, generator=None, latents: Optional[torch.Tensor] = None,
+                 prompt_embeds: Optional[torch.Tensor] = None, negative_prompt_embeds: Optional[torch.Tensor] = None,
+                 pooled_prompt_embeds: Optional[torch.Tensor] = None,
+                 negative_pooled_prompt_embeds: Optional[torch.Tensor] = None, output_type: Optional[str] = "pil",
+                 return_dict: bool = True, callback=None, callback_steps: int = 1,
+                 cross_attention_kwargs: Optional[Dict[str, Any]] = None, guidance_rescale: float = 0.0,
+                 original_size: Optional[Tuple[int, int]] = None, crops_coords_top_left: Tuple[int, int] = (0, 0),
+                 target_size: Optional[Tuple[int, int]] = None, negative_original_size=None,
+                 negative_crops_coords_top_left=(0, 0), negative_target_size=None,
+                 control_guidance_start: float = 0.0, control_guidance_end: float = 1.0, aesthetic_score: float = 6.0,
+                 negative_aesthetic_score: float = 2.5, **ignored):
+        """The img2img parameters plus `mask_image`, `height` and `width` (default unet sample_size * 8, multiples of
+        8).  `strength` = 1.0 starts from pure noise; the source latents are still used by the blend.  `latents` is not
+        used; `aesthetic_score*` are accepted and ignored, as in img2img."""
+        if image is None or mask_image is None:
+            raise ValueError("inpainting needs a source `image` and a `mask_image`")
+        height = height or self.default_sample_size * self.vae_scale_factor
+        width = width or self.default_sample_size * self.vae_scale_factor
+        if height % self.vae_scale_factor or width % self.vae_scale_factor:
+            raise ValueError(f"`height` and `width` have to be divisible by 8 but are {height} and {width}.")
+        t_start = self._check_edit_args(strength, num_inference_steps, callback, callback_steps)
+        do_classifier_free_guidance = guidance_scale > 1.0
+        embeds = self.encode_prompt(prompt, prompt_2, None, num_images_per_prompt, do_classifier_free_guidance,
+                                    negative_prompt, negative_prompt_2, prompt_embeds, negative_prompt_embeds,
+                                    pooled_prompt_embeds, negative_pooled_prompt_embeds)
+        self.scheduler.set_timesteps(num_inference_steps)
+        lat, inpaint = self.prepare_inpaint_latents(image, mask_image, embeds[0].shape[0], generator, height, width,
+                                                    t_start, strength == 1.0)
+        return self._denoise_and_decode(
+            lat, t_start, num_inference_steps, embeds, guidance_scale=guidance_scale, denoising_end=denoising_end,
+            guidance_rescale=guidance_rescale, original_size=original_size or (height, width),
+            crops_coords_top_left=crops_coords_top_left, target_size=target_size or (height, width),
+            negative_original_size=negative_original_size, negative_crops_coords_top_left=negative_crops_coords_top_left,
+            negative_target_size=negative_target_size, control_guidance_start=control_guidance_start,
+            control_guidance_end=control_guidance_end, callback=callback, callback_steps=callback_steps,
+            output_type=output_type, return_dict=return_dict, inpaint=inpaint)
